@@ -6,13 +6,14 @@ of one batched frame step.  Headline workload = configs[1]: 4,096 concurrent 16 
 every stream by `--frames-per-step` 512-sample frames (hop 512).  Weak scaling: streams per GPU fixed.
 
   python bench.py [--gpus N] [--steps K] [--warmup W]              our arm
+  python bench.py [...] --dump-outputs DIR                          ... and DIR/<name>.npy = what its last timed step returned
   python bench.py --impl reference [...]                            CPU arm (oracle port, all host threads)
 
 One JSON line on stdout (rank 0).  Besides the contract's keys (DESIGN.md "Measurement"):
-  value / ms_per_step      median over `repeats` timed regions of exactly K steps each (barrier + synchronize on both
-                           sides of every region, max over ranks per region); value_min / value_max beside it
+  value / ms_per_step      one timed region of exactly K steps (barrier + synchronize on both sides, max over ranks) after
+                           0.5 s of untimed steps, an engine reset and max(W, input pool size) warm-up steps
   e2e                      the public host-buffer call with the wire format (int16 PCM, CVAD_PCM_S16_32767) in pinned host
-                           buffers, H2D + D2H inside the timed region; e2e.f32 = the same with float32 PCM
+                           buffers, H2D + D2H inside the timed region of K steps; e2e.f32 = the same with float32 PCM
   value_fp32               the same workload on the FP32-FMA build of the kernels (same-precision anchor)
   extra                    the other configurations of BASELINE.json, each with its own roofline:
                              configs2  v4 behind the 8 kHz resampler, 16,384 streams (N = 1 only)
@@ -30,6 +31,7 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 from collections import deque
@@ -162,7 +164,9 @@ class ClockSampler:
 def cpu_port(native=True):
     sys.path.insert(0, str(ROOT / "oracle"))
     from vad_oracle import RefLib, RefV5, v5_blob
-    lib = RefLib(native=native)
+    # compiled for this host at run time, so outside the tree (which may be read-only); the loaded library outlives its file
+    with tempfile.TemporaryDirectory(prefix="cvad_bench_") as tmp:
+        lib = RefLib(native=native, build_dir=tmp)
     blob = v5_blob(str(ROOT / "cutter-vad_b200" / "real_time_vad" / "models" / "silero_vad_v5.onnx"))
     return lib, RefV5(blob, lib)
 
@@ -329,48 +333,83 @@ class Workload:
     def audio_s_per_step(self):
         return self.n * self.F * 0.032
 
+    def outputs(self):
+        """What a caller of the last device step received: probabilities [n][F], flags [n][F] and the event records
+        [events][stream, slot, frame, kind, stream_frame], sorted (the kernel appends events in no fixed order)."""
+        n_ev = min(int(self.d_nev.item()), self.max_events)
+        rec = np.dtype([("stream", "<i4"), ("slot", "<i4"), ("frame", "<i4"), ("kind", "<i4"), ("stream_frame", "<i8")])
+        ev = self.d_events[:n_ev * rec.itemsize].cpu().numpy().view(rec)
+        ev = np.stack([ev[k].astype(np.float64) for k in rec.names], axis=1).reshape(n_ev, len(rec.names))
+        ev = ev[np.lexsort(ev.T[::-1])]
+        return self.d_probs.cpu().numpy(), self.d_flags.cpu().numpy(), ev
 
-def time_device(torch, dist, world, eng, wl, stream, steps, warmup, min_repeats=15, target_s=1.5, max_repeats=2000):
-    """`value` leg: inputs resident in HBM, cvad_step_device, CUDA events on the engine's stream.  The region of exactly
-    `steps` steps is timed `repeats` times (barrier + synchronize on both sides of each); per region the max over ranks.
-    -> dict(region_ms [repeats], launches per region, per-step latency p50 / p99, per-kernel ms from a separate pass)"""
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, outputs):
+    """DIR/<name>.npy: probs, flags (float32), events and streams (float64, the stream index of each row).  Over DUMP_BYTES
+    in the worst case (one event per stream and frame) the rows are a fixed seeded sample of the streams."""
+    probs, flags, ev = outputs
+    n, F = probs.shape
+    rows = np.arange(n)
+    per_row = 8 * F + 8 + 40 * F
+    if n * per_row > DUMP_BYTES - 4096:                     # (room for the four .npy headers)
+        k = (DUMP_BYTES - 4096) // per_row
+        rows = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+        ev = ev[np.isin(ev[:, 0], rows)]
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    np.save(d / "probs.npy", probs[rows].astype(np.float32))
+    np.save(d / "flags.npy", flags[rows].astype(np.float32))
+    np.save(d / "events.npy", ev)
+    np.save(d / "streams.npy", rows.astype(np.float64))
+
+
+def settle(step, barrier, seconds=0.5):
+    """Untimed steps for `seconds` of wall time: GPU clocks and host threads reach the state of a service under sustained
+    load.  The caller resets the engine afterwards, so that what is timed and returned depends on the arguments only."""
+    i, t_end = 0, time.perf_counter() + seconds
+    while time.perf_counter() < t_end:
+        step(i)
+        i += 1
+    barrier()
+
+
+def time_device(torch, dist, world, eng, wl, stream, steps, warmup, keep_outputs=False):
+    """`value` leg: inputs resident in HBM, cvad_step_device, CUDA events on the engine's stream.  After `warmup` untimed
+    steps, ONE region of exactly `steps` steps is timed (barrier + synchronize on both sides; the max over ranks).
+    -> dict(region_ms, launches in the region, per-step latency p50 / p99, per-kernel ms from a separate pass, and with
+    `keep_outputs` what the region's last step returned)"""
     def barrier():
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
 
+    settle(lambda i: eng.step_device(wl.dargs[i % wl.pool_n]), barrier)
     eng.reset()
+    # the warm-up steps every buffer of the pool at least once: a buffer's first read pays address-translation misses
+    # that a running service never sees
+    warmup = max(warmup, wl.pool_n)
     for i in range(warmup):
         eng.step_device(wl.dargs[i % wl.pool_n])
     eng.sync()
     barrier()
-
-    def region(k0):
-        e0 = torch.cuda.Event(enable_timing=True)
-        e1 = torch.cuda.Event(enable_timing=True)
-        l0 = eng.launch_count()
-        with torch.cuda.stream(stream):
-            e0.record(stream)
-            for i in range(steps):
-                eng.step_device(wl.dargs[(k0 + i) % wl.pool_n])
-            e1.record(stream)
-        barrier()
-        return e0.elapsed_time(e1), eng.launch_count() - l0
-
-    first_ms, launches = region(warmup)
-    repeats = int(min(max_repeats, max(min_repeats, target_s * 1e3 / max(first_ms, 1e-3))))
-    if world > 1:                                            # every rank must run the same number of barriers
-        r = torch.tensor([repeats], dtype=torch.int64, device=f"cuda:{wl.local}")
-        dist.all_reduce(r, op=dist.ReduceOp.MIN)
-        repeats = int(r[0])
-    ms = [first_ms]
-    for r in range(1, repeats):
-        t, _ = region(warmup + r * steps)
-        ms.append(t)
-    ms_t = torch.tensor(ms, dtype=torch.float64, device=f"cuda:{wl.local}")
+    e0 = torch.cuda.Event(enable_timing=True)
+    e1 = torch.cuda.Event(enable_timing=True)
+    l0 = eng.launch_count()
+    with torch.cuda.stream(stream):
+        e0.record(stream)
+        for i in range(steps):
+            eng.step_device(wl.dargs[(warmup + i) % wl.pool_n])
+        e1.record(stream)
+    barrier()
+    launches = eng.launch_count() - l0
+    outputs = wl.outputs() if keep_outputs else None
+    ms_t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=f"cuda:{wl.local}")
     if world > 1:
         dist.all_reduce(ms_t, op=dist.ReduceOp.MAX)
-    region_ms = ms_t.cpu().numpy()
+    region_ms = float(ms_t[0])
     # per-kernel durations for the roofline: the same K steps again with events around the kernels
     # (kept out of the passes above: events between the kernels would serialise their overlap)
     eng.set_timing(True)
@@ -381,7 +420,7 @@ def time_device(torch, dist, world, eng, wl, stream, steps, warmup, min_repeats=
     fe_ms, rec_ms, n_timed = eng.read_timing()
     eng.set_timing(False)
     lat = []
-    for i in range(min(max(steps, 50), 200)):
+    for i in range(steps):
         a0 = torch.cuda.Event(enable_timing=True)
         a1 = torch.cuda.Event(enable_timing=True)
         a0.record(stream)
@@ -389,18 +428,16 @@ def time_device(torch, dist, world, eng, wl, stream, steps, warmup, min_repeats=
         a1.record(stream)
         a1.synchronize()
         lat.append(a0.elapsed_time(a1))
-    return {"region_ms": region_ms, "launches": int(launches), "repeats": repeats,
+    return {"region_ms": region_ms, "launches": int(launches), "outputs": outputs, "warmup": warmup,
             "fe_ms": fe_ms / max(n_timed, 1), "rec_ms": rec_ms / max(n_timed, 1),
             "p50_step_ms": float(np.percentile(lat, 50)), "p99_step_ms": float(np.percentile(lat, 99))}
 
 
-def time_e2e(torch, dist, world, eng, wl, steps, warmup, pcm: str, depth=4, min_s=0.5):
+def time_e2e(torch, dist, world, eng, wl, steps, warmup, pcm: str, depth=4):
     """`e2e` leg: the public host-buffer call (StreamEngine.submit / collect -> cvad_step_submit / _collect) with `depth`
-    steps in flight; every step's H2D of its inputs and D2H of its results is inside the timed region (wall clock, max
-    over ranks).  The K-step region is repeated until `min_s` seconds have been measured; the median region counts."""
+    steps in flight; every step's H2D of its inputs and D2H of its results is inside the timed region of exactly `steps`
+    steps (wall clock, max over ranks).  A short region mostly measures the fill and drain of the pipeline."""
     capi = wl.capi
-    # a region shorter than ~100 steps mostly measures the fill and drain of the four-deep pipeline (20 steps: -5 %)
-    steps = max(int(steps), 100)
     pool = [t.numpy() for t in (wl.host_s16 if pcm == "s16" else wl.host_f32)]
     kw = dict(wl.rate_kw)
     if pcm == "s16":
@@ -411,46 +448,38 @@ def time_e2e(torch, dist, world, eng, wl, steps, warmup, pcm: str, depth=4, min_
             dist.barrier()
         torch.cuda.synchronize()
 
-    eng.reset()
-    for i in range(warmup):
-        eng.step(pool[i % len(pool)], **kw)
-    barrier()
-    regions, events, k0 = [], 0, 0
-    t_all = time.perf_counter()
-    while True:
+    def pipelined(k):
         inflight = deque()
-        barrier()
-        t0 = time.perf_counter()
-        for i in range(steps):
-            inflight.append(eng.submit(pool[(k0 + i) % len(pool)], **kw))
+        for i in range(k):
+            inflight.append(eng.submit(pool[i % len(pool)], **kw))
             if len(inflight) == depth:
                 r = inflight.popleft().collect()
         while inflight:
             r = inflight.popleft().collect()
-        torch.cuda.synchronize()
-        dt = time.perf_counter() - t0
-        events = len(r.events)
-        t = torch.tensor([dt, float(time.perf_counter() - t_all >= min_s and len(regions) + 1 >= 5)],
-                         dtype=torch.float64, device=f"cuda:{wl.local}")
-        if world > 1:
-            dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        regions.append(float(t[0]))
-        k0 += steps
-        if float(t[1]) > 0 or len(regions) >= 400:
-            break
+        return r
+
+    settle(lambda i: pipelined(32), barrier)
+    eng.reset()
+    pipelined(max(warmup, depth))          # the warm-up runs every lane of the pipeline the timed region uses
+    barrier()
+    t0 = time.perf_counter()
+    r = pipelined(steps)
+    torch.cuda.synchronize()
+    t = torch.tensor([time.perf_counter() - t0], dtype=torch.float64, device=f"cuda:{wl.local}")
+    if world > 1:
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+    dt = float(t[0])
+    events = len(r.events)
     # one call at a time: latency distribution of the blocking form
     lat = []
-    for i in range(min(max(steps, 50), 200)):
+    for i in range(steps):
         t1 = time.perf_counter()
         eng.step(pool[i % len(pool)], **kw)
         lat.append(time.perf_counter() - t1)
-    med = float(np.median(regions))
     es = 2 if pcm == "s16" else 4
-    return {"value": wl.audio_s_per_step * steps * world / med, "unit": "audio-s/s",
+    return {"value": wl.audio_s_per_step * steps * world / dt, "unit": "audio-s/s",
             "h2d_bytes_per_step": wl.n * wl.step_samples * es, "d2h_bytes_per_step": wl.n * wl.F * 5 + wl.n * 4 + 4,
-            "ms_per_step": 1e3 * med / steps, "repeats": len(regions), "region_steps": steps,
-            "value_min": wl.audio_s_per_step * steps * world / max(regions),
-            "value_max": wl.audio_s_per_step * steps * world / min(regions),
+            "ms_per_step": 1e3 * dt / steps,
             "p50_call_ms": 1e3 * float(np.percentile(lat, 50)), "p99_call_ms": 1e3 * float(np.percentile(lat, 99)),
             "pcm": ("int16 (the websocket wire format, vad_websocket_server.py:341), / 32767.0f in the frame loader"
                     if pcm == "s16" else "float32"),
@@ -614,19 +643,20 @@ def run_ours(args):
     sampler.start()
     time.sleep(0.12)
     c_lo = sampler.mark()
-    dev = time_device(torch, dist, world, eng, wl, stream, args.steps, args.warmup)
+    dev = time_device(torch, dist, world, eng, wl, stream, args.steps, args.warmup, keep_outputs=bool(args.dump_outputs))
     c_hi = sampler.mark()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dev["outputs"])
     e2e = time_e2e(torch, dist, world, eng, wl, args.steps, args.warmup, "s16")
     e2e_f32 = time_e2e(torch, dist, world, eng, wl, args.steps, args.warmup, "f32")
     h2d_gbs = pinned_copy_rate(torch, wl)
     eng.close()
 
-    region = dev["region_ms"]
-    med_ms = float(np.median(region))
+    region_ms = dev["region_ms"]
     total_audio = wl.audio_s_per_step * args.steps * world
-    value = total_audio / (med_ms * 1e-3)
+    value = total_audio / (region_ms * 1e-3)
     frames_per_step = n * F
-    step_ms = med_ms / args.steps
+    step_ms = region_ms / args.steps
 
     extras = {}
     value_fp32 = None
@@ -637,11 +667,11 @@ def run_ours(args):
         e32.set_math("fp32")
         e32.configure(enable_denoising=True)
         e32.set_stream(stream.cuda_stream)
-        d32 = time_device(torch, dist, world, e32, wl, stream, args.steps, args.warmup, target_s=0.5)
+        d32 = time_device(torch, dist, world, e32, wl, stream, args.steps, args.warmup)
         e32.close()
-        m32 = float(np.median(d32["region_ms"]))
+        m32 = d32["region_ms"]
         value_fp32 = {"value": total_audio / (m32 * 1e-3), "unit": "audio-s/s", "ms_per_step": m32 / args.steps,
-                      "math": "fp32 (packed FP32 FMA on the CUDA cores, ascending-k accumulation)", "repeats": d32["repeats"],
+                      "math": "fp32 (packed FP32 FMA on the CUDA cores, ascending-k accumulation)",
                       "roofline": simple_roofline("v5_frontend_kernel + v5_recurrent_kernel", "fp32_ffma", FLOP_V5, frames_per_step,
                                                   m32 / args.steps, peak_fp32, peak_fp32_src)}
     del wl
@@ -653,15 +683,15 @@ def run_ours(args):
         e3 = StreamEngine("v5", max_streams=8192, device=local)
         e3.configure(enable_denoising=True)
         e3.set_stream(stream.cuda_stream)
-        d3 = time_device(torch, dist, world, e3, w3, stream, args.steps, args.warmup, target_s=0.5)
-        x3 = time_e2e(torch, dist, world, e3, w3, args.steps, args.warmup, "s16", min_s=0.4)
+        d3 = time_device(torch, dist, world, e3, w3, stream, args.steps, args.warmup)
+        x3 = time_e2e(torch, dist, world, e3, w3, args.steps, args.warmup, "s16")
         e3.close()
-        m3 = float(np.median(d3["region_ms"]))
+        m3 = d3["region_ms"]
         flop3 = FLOP_V5 + (FLOP_RESAMPLE[24000] + FLOP_RESAMPLE[48000]) // 2
         extras["configs3"] = {
             "config": workload_config("v5", 8192, 1, 48000, True), "n_gpus": world,
             "value": w3.audio_s_per_step * args.steps * world / (m3 * 1e-3), "unit": "audio-s/s", "ms_per_step": m3 / args.steps,
-            "p99_step_ms": d3["p99_step_ms"], "repeats": d3["repeats"], "gpu_launches": d3["launches"],
+            "p99_step_ms": d3["p99_step_ms"], "gpu_launches": d3["launches"],
             "e2e": x3,
             "roofline": simple_roofline("rate_lists + 2 x resample_fft_kernel + v5tc_frontend_kernel<FUSED,H16>", "tensor", flop3,
                                         8192, m3 / args.steps, peak_bf16, peak_bf16_src)}
@@ -674,13 +704,12 @@ def run_ours(args):
         e2 = StreamEngine("v4", max_streams=16384, device=local)
         e2.configure(enable_denoising=True)
         e2.set_stream(stream.cuda_stream)
-        k2 = max(args.steps // 4, 5)
-        d2 = time_device(torch, dist, world, e2, w2, stream, k2, args.warmup, target_s=0.5)
-        m2 = float(np.median(d2["region_ms"])) / k2
+        d2 = time_device(torch, dist, world, e2, w2, stream, args.steps, args.warmup)
+        m2 = d2["region_ms"] / args.steps
         extras["configs2"] = {
-            "config": workload_config("v4", 16384, 1, 8000), "math": e2.math, "n_gpus": 1, "steps": k2,
+            "config": workload_config("v4", 16384, 1, 8000), "math": e2.math, "n_gpus": 1,
             "value": w2.audio_s_per_step / (m2 * 1e-3), "unit": "audio-s/s", "ms_per_step": m2,
-            "p99_step_ms": d2["p99_step_ms"], "repeats": d2["repeats"], "gpu_launches": d2["launches"],
+            "p99_step_ms": d2["p99_step_ms"], "gpu_launches": d2["launches"],
             "kernel_ms": {"frontend_kernels": d2["fe_ms"], "v4_recurrent_kernel": d2["rec_ms"]},
             "roofline": simple_roofline("resample_fft<1> + v4_stft_fft + v4tc_stft<CORR> + v4_frontend + v4_recurrent", "fp32_ffma",
                                         FLOP_V4 + FLOP_RESAMPLE[8000], 16384, m2, peak_fp32, peak_fp32_src)}
@@ -751,7 +780,7 @@ def run_ours(args):
             "peak_source": peak_bf16_src if tc else peak_fp32_src,
             "algorithmic_flop_per_frame": flop_fe, "frames_per_launch": frames_per_step,
             "avg_launch_ms": fe_s * 1e3, "isolated_launch_ms": isolated_ms,
-            "kernel_timing": ("avg_launch_ms = median timed region (CUDA events on the engine's stream) / launches: a region holds "
+            "kernel_timing": ("avg_launch_ms = timed region (CUDA events on the engine's stream) / launches: the region holds "
                               "nothing but this kernel's K launches, chained by programmatic dependent launch; "
                               "isolated_launch_ms = separate pass with events around every launch (no overlap)" if chained else
                               "separate pass over the same K steps with a CUDA event between the kernels"),
@@ -770,7 +799,7 @@ def run_ours(args):
             roofline["executed_bf16_tflops"] = products * fe_tflops
             roofline["executed_frac"] = products * fe_tflops / peak_bf16
         cpu = None if args.skip_cpu else cpu_baseline_sample(n)
-        e2e["f32"] = {k: e2e_f32[k] for k in ("value", "h2d_bytes_per_step", "ms_per_step", "value_min", "value_max", "repeats")}
+        e2e["f32"] = {k: e2e_f32[k] for k in ("value", "h2d_bytes_per_step", "ms_per_step")}
         e2e["pinned_h2d_gbs"] = h2d_gbs
         e2e["transfer_bound_value"] = transfer_bound(n, F, rate, mixed, world, h2d_gbs)
         e2e["numa"] = numa
@@ -786,10 +815,8 @@ def run_ours(args):
             "data": "synthetic", "config": workload_config(model, n, F, rate, mixed),
             "math": math,
             "l2": f"inputs cycle through a pool of distinct step buffers totalling {round(dev_pool_mb(n, F, rate, mixed))} MB (> 126 MB L2)",
-            "repeats": dev["repeats"],
-            "value_min": total_audio / (float(region.max()) * 1e-3), "value_max": total_audio / (float(region.min()) * 1e-3),
-            "timing": f"value = K steps / median of {dev['repeats']} timed regions of exactly K = {args.steps} steps each "
-                      "(barrier + synchronize around every region, max over ranks per region)",
+            "timing": f"value = K steps / one timed region of exactly K = {args.steps} steps after {dev['warmup']} untimed ones "
+                      "(W, and at least one pass over the input pool; barrier + synchronize around the region, max over ranks)",
             "p99_step_ms": dev["p99_step_ms"], "p50_step_ms": dev["p50_step_ms"],
             "frames_per_s": value / 0.032,
             "roofline": roofline,
@@ -849,7 +876,14 @@ def main():
     ap.add_argument("--model", choices=["v5", "v4"], default="v5", help="v5 = headline (configs[1]); v4 = configs[2]")
     ap.add_argument("--src-rate", type=int, default=16000, choices=[8000, 16000, 24000, 48000],
                     help="source rate of the synthetic streams; != 16000 adds the GPU resampler (configs[2..3])")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline configuration returned (rank 0's streams) as "
+                         "DIR/<name>.npy; the inputs depend only on the arguments, so two builds can be compared")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU arm computed: not with --impl reference")
     if args.math is None:
         args.math = "tc16" if args.model == "v5" else "fft"
     args.warmup = max(args.warmup, 3)

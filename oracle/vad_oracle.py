@@ -135,13 +135,13 @@ def v4_blob(onnx_path: str) -> np.ndarray:
 # C restatement: build + bind
 # ----------------------------------------------------------------------------
 
-def build_ref_lib(native: bool = False, force: bool = False) -> str:
-    """Compile oracle/silero_ref.c.  `native=True` (bench's CPU-baseline leg, run on
+def build_ref_lib(native: bool = False, force: bool = False, build_dir: str = BUILD_DIR) -> str:
+    """Compile oracle/silero_ref.c into `build_dir`.  `native=True` (bench's CPU-baseline leg, run on
     the GPU box's host) uses -march=native into a separate file; the default is a
     portable AVX2+FMA build that may travel between machines of this image."""
-    os.makedirs(BUILD_DIR, exist_ok=True)
+    os.makedirs(build_dir, exist_ok=True)
     tag = "native" if native else "avx2"
-    so = os.path.join(BUILD_DIR, f"libsilero_ref_{tag}.so")
+    so = os.path.join(build_dir, f"libsilero_ref_{tag}.so")
     src = os.path.join(_HERE, "silero_ref.c")
     if (not force) and os.path.exists(so) and os.path.getmtime(so) >= os.path.getmtime(src):
         return so
@@ -159,8 +159,8 @@ def _fp(a: np.ndarray):
 
 
 class RefLib:
-    def __init__(self, native: bool = False):
-        self.path = build_ref_lib(native=native)
+    def __init__(self, native: bool = False, build_dir: str = BUILD_DIR):
+        self.path = build_ref_lib(native=native, build_dir=build_dir)
         L = ctypes.CDLL(self.path)
         L.sref_v5_create.restype = ctypes.c_void_p
         L.sref_v5_create.argtypes = [_f32p]

@@ -136,27 +136,31 @@ def test_4096_streams_2000_chained_steps_no_drift(engine_factory, ref_v5, ref_li
     flags_d = torch.full((T, n), 255, dtype=torch.uint8, device=cu)
     nev_d = torch.zeros((T,), dtype=torch.int32, device=cu)
     ev_d = torch.zeros((T, n * 24), dtype=torch.uint8, device=cu)
-    # the engine runs on torch's stream so that the per-step gather of the 16 replicas is ordered with the steps
-    eng.set_stream(torch.cuda.current_stream().cuda_stream)
+    # the engine and the per-step gather of the 16 replicas share one torch stream, so that they are ordered.  Not torch's
+    # default stream: its handle is 0, which set_stream takes as "the engine's own stream", unordered with the gather.
+    stream = torch.cuda.Stream(device=cu)
+    stream.wait_stream(torch.cuda.current_stream())
+    eng.set_stream(stream.cuda_stream)
     try:
-        bufs = [torch.empty((n, 512), dtype=torch.float32, device=cu) for _ in range(4)]
-        for j in range(T):
-            x = bufs[j % 4]
-            x.view(n // distinct, distinct, 512).copy_(base_d[:, j * 512:(j + 1) * 512].unsqueeze(0).expand(n // distinct, -1, -1))
-            a = capi.StepArgs()
-            a.n_streams = n
-            a.audio = x.data_ptr()
-            a.pcm_format = capi.PCM_F32
-            a.stream_stride = 512
-            a.max_frames = 1
-            a.frame_len = a.hop = 512
-            a.src_rate = 16000
-            a.probs_out = probs_d[j].data_ptr()
-            a.flags_out = flags_d[j].data_ptr()
-            a.events_out = ev_d[j].data_ptr()
-            a.max_events = n
-            a.n_events_out = nev_d[j:j + 1].data_ptr()
-            eng.step_device(a)
+        with torch.cuda.stream(stream):
+            bufs = [torch.empty((n, 512), dtype=torch.float32, device=cu) for _ in range(4)]
+            for j in range(T):
+                x = bufs[j % 4]
+                x.view(n // distinct, distinct, 512).copy_(base_d[:, j * 512:(j + 1) * 512].unsqueeze(0).expand(n // distinct, -1, -1))
+                a = capi.StepArgs()
+                a.n_streams = n
+                a.audio = x.data_ptr()
+                a.pcm_format = capi.PCM_F32
+                a.stream_stride = 512
+                a.max_frames = 1
+                a.frame_len = a.hop = 512
+                a.src_rate = 16000
+                a.probs_out = probs_d[j].data_ptr()
+                a.flags_out = flags_d[j].data_ptr()
+                a.events_out = ev_d[j].data_ptr()
+                a.max_events = n
+                a.n_events_out = nev_d[j:j + 1].data_ptr()
+                eng.step_device(a)
         eng.sync()
         torch.cuda.synchronize()
     finally:

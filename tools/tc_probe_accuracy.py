@@ -1,5 +1,6 @@
 import sys, numpy as np, ctypes as C
-sys.path.insert(0, '/root/repo/cutter-vad_b200')
+from pathlib import Path
+sys.path.insert(0, str(Path(__file__).resolve().parents[1] / 'cutter-vad_b200'))
 from real_time_vad.engine import capi
 L = capi.dev_lib()
 def bf16_bits(x):

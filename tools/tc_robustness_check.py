@@ -1,6 +1,6 @@
 import sys, numpy as np
 from pathlib import Path
-ROOT = Path('/root/repo')
+ROOT = Path(__file__).resolve().parents[1]
 for p in (ROOT / "cutter-vad_b200", ROOT / "oracle", ROOT / "tests"): sys.path.insert(0, str(p))
 from conftest import synth_streams, V5_ONNX
 from real_time_vad.engine.stream_engine import StreamEngine
