@@ -25,7 +25,7 @@ def _fresh(out: Path) -> bool:
 
 def build(force: bool = False, verbose: bool = False) -> Path:
     nvcc = os.environ.get("NVCC", "nvcc")
-    extra = os.environ.get("CVAD_NVCC_EXTRA", "").split()          # experiments, e.g. -DCVAD_H16_MERGE=1
+    extra = os.environ.get("CVAD_NVCC_EXTRA", "").split()          # extra nvcc flags for experimental builds
     for src, out in ((SRC, OUT), (DEV_SRC, DEV_OUT)):
         if not force and _fresh(out):
             continue

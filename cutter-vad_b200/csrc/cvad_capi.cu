@@ -51,7 +51,6 @@ struct cvad_engine {
     int math = CVAD_MATH_FP32;
     bool v4_t2 = false;                // CVAD_MODEL_V4_8K: two LSTM time steps per frame
     bool fuse_single_frame = true;     // CVAD_FUSE=0 keeps the two-kernel form for one-frame steps (measurement)
-    bool h16_multi = true;             // CVAD_H16_MULTI=0: multi-frame steps of CVAD_MATH_TC16 run the BF16-split kernels
     bool chain_steps = true;           // CVAD_CHAIN=0: device-pointer steps are not chained (memsets + event record per step; measurement)
     unsigned char *w_fe_tc = nullptr, *w_rec_tc = nullptr;
     unsigned char *w_fe_h = nullptr, *w_rec_h = nullptr;   // CVAD_MATH_TC16: two FP16 parts, per-layer scale
@@ -924,7 +923,7 @@ int launch_step(cvad_engine *e, const cvad_step_args *a, unsigned int *d_status,
             return CVAD_OK;
         }
         if (chain) return fail(e, CVAD_E_INVALID, "internal: chained step outside the fused one-frame path");
-        const bool h16 = e->math == CVAD_MATH_TC16 && !d_dbg && e->h16_multi;
+        const bool h16 = e->math == CVAD_MATH_TC16 && !d_dbg;
         if (h16) {
             p.w_fe_h = e->w_fe_h; p.w_rec_h = e->w_rec_h;
             std::memcpy(p.tc16_inv_w, e->tc16_inv_w, sizeof(p.tc16_inv_w));
@@ -1388,8 +1387,6 @@ int cvad_create(const float *weights, size_t n_weight_floats, int model_version,
                   : (m && std::strcmp(m, "tc") == 0) ? CVAD_MATH_TC : CVAD_MATH_TC16;
         const char *fz = std::getenv("CVAD_FUSE");
         e->fuse_single_frame = !(fz && std::strcmp(fz, "0") == 0);
-        const char *hm = std::getenv("CVAD_H16_MULTI");
-        e->h16_multi = !(hm && std::strcmp(hm, "0") == 0);
         const char *ch = std::getenv("CVAD_CHAIN");
         e->chain_steps = !(ch && std::strcmp(ch, "0") == 0);
     }
@@ -1421,10 +1418,10 @@ int cvad_create(const float *weights, size_t n_weight_floats, int model_version,
         int rc;
         if ((rc = upload(e, &e->w_fe_tc, T))) return bail(rc);
         // v4 feeds log(1 + 2^20 |STFT|) into the network, which amplifies the tensor cores' (truncating) FP32
-        // accumulation on weak bins: FP32 FMA stays the default for v4, the tensor-core STFT is opt-in
-        // since then: the STFT as a double-precision FFT plus a tensor-core correction for the basis' float32 rounding
-        // (CVAD_MATH_FFT) is both faster and closer to the float64 evaluation of the graph than either; it is the
-        // default whenever the blob's basis is Hann x DFT-256 (true for both sub-models of the reference's file)
+        // accumulation on weak bins, so the tensor-core STFT (CVAD_MATH_TC) is opt-in although it is the fastest v4 path.
+        // The STFT as a double-precision FFT plus a tensor-core correction for the basis' float32 rounding
+        // (CVAD_MATH_FFT) is the closest to the float64 evaluation of the graph of the three; it is the default
+        // whenever the blob's basis is Hann x DFT-256 (true for both sub-models of the reference's file)
         std::vector<unsigned char> C;
         const double worst = pack_v4_stft_corr(weights, fftT.data(), C);
         e->v4_fft_ok = worst <= 2.0e-7;

@@ -344,11 +344,6 @@ __device__ __forceinline__ void store_parts2_h(unsigned char *base, uint32_t ps,
     *reinterpret_cast<unsigned short *>(db) = (unsigned short)(w0 >> 16);
     *reinterpret_cast<unsigned short *>(db + ps) = (unsigned short)(w1 >> 16);
 }
-// CVAD_H16_MERGE=1 (experiment): the three products of the FP16 split accumulate in ONE accumulator, corrections first
-#ifndef CVAD_H16_MERGE
-#define CVAD_H16_MERGE 0
-#endif
-constexpr bool kH16Merge = CVAD_H16_MERGE != 0;
 // ---- B operands MN-major SWIZZLE_64B (fused FP16 build, every operand an epilogue writes: MAG, E0, E1, E2, X, H)
 // An epilogue thread owns ONE channel (its TMEM lane = the next layer's k) and EIGHT consecutive streams: with N as the
 // contiguous dimension those are one 16-byte chunk per part and time column -- 2 STS.128 where the K-major layout took
@@ -372,10 +367,10 @@ __device__ __forceinline__ void issue_split_mn(int wp, uint32_t a_addr, uint32_t
     for (int ks = 0; ks < 4; ++ks) {
         const uint32_t fresh = (first && ks == 0) ? 0u : 1u;
         if (wp == 0) {
-            tc::mma_bf16(kH16Merge ? d_main : d_corr, ad + ks * 2, bd1 + ks * kst, idesc, fresh);
-            tc::mma_bf16(d_main, ad + ks * 2, bd0 + ks * kst, idesc, kH16Merge ? 1u : fresh);
+            tc::mma_bf16(d_corr, ad + ks * 2, bd1 + ks * kst, idesc, fresh);
+            tc::mma_bf16(d_main, ad + ks * 2, bd0 + ks * kst, idesc, fresh);
         } else {
-            tc::mma_bf16(kH16Merge ? d_main : d_corr, ad + ks * 2, bd0 + ks * kst, idesc, 1u);
+            tc::mma_bf16(d_corr, ad + ks * 2, bd0 + ks * kst, idesc, 1u);
         }
     }
 }
@@ -432,14 +427,6 @@ __host__ __device__ __forceinline__ void fe_slot_h(int s, uint32_t &off, uint32_
 constexpr size_t kRecStreamBytesH = (size_t)32 * 16384;       // gate x kb 0..3 x part 0..1
 constexpr int kFusedSlotsPerTileH = 16 + kFeSlotsPerTileH + 16;
 constexpr uint32_t kColIh = 0;                                // TMEM columns of the W_ih . x accumulators (64 per gate; free after encoder.3)
-__device__ __forceinline__ void tmem_ld8_corr(uint32_t taddr, float (&v)[8]) {
-    if (kH16Merge) {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) v[i] = 0.f;
-    } else {
-        tmem_ld8(taddr, v);
-    }
-}
 // MMAs of one weight tile (part wp) for one 64-element K block, FP16 split: w0.x0 -> d_main, w0.x1 and w1.x0 -> d_corr
 __device__ __forceinline__ void issue_split_h(int wp, uint32_t a_addr, uint32_t b0, uint32_t ps, uint32_t d_main,
                                               uint32_t d_corr, uint32_t idesc, bool first) {
@@ -449,10 +436,10 @@ __device__ __forceinline__ void issue_split_h(int wp, uint32_t a_addr, uint32_t 
     for (int ks = 0; ks < 4; ++ks) {
         const uint32_t fresh = (first && ks == 0) ? 0u : 1u;
         if (wp == 0) {
-            tc::mma_bf16(kH16Merge ? d_main : d_corr, ad + ks * 2, bd1 + ks * 2, idesc, fresh);
-            tc::mma_bf16(d_main, ad + ks * 2, bd0 + ks * 2, idesc, kH16Merge ? 1u : fresh);
+            tc::mma_bf16(d_corr, ad + ks * 2, bd1 + ks * 2, idesc, fresh);
+            tc::mma_bf16(d_main, ad + ks * 2, bd0 + ks * 2, idesc, fresh);
         } else {
-            tc::mma_bf16(kH16Merge ? d_main : d_corr, ad + ks * 2, bd0 + ks * 2, idesc, 1u);
+            tc::mma_bf16(d_corr, ad + ks * 2, bd0 + ks * 2, idesc, 1u);
         }
     }
 }
@@ -1093,8 +1080,8 @@ __global__ void __launch_bounds__(kThreadsTC, 1) v5tc_frontend_kernel(const V5St
                     float mr[8], mi[8], cr[8], ci[8];
                     tmem_ld8(lane_addr + kColMain + c0, mr);
                     tmem_ld8(lane_addr + kColMain + 96 + c0, mi);
-                    tmem_ld8_corr(lane_addr + kColCorr + c0, cr);
-                    tmem_ld8_corr(lane_addr + kColCorr + 96 + c0, ci);
+                    tmem_ld8(lane_addr + kColCorr + c0, cr);
+                    tmem_ld8(lane_addr + kColCorr + 96 + c0, ci);
                     tmem_wait_ld();
 #pragma unroll
                     for (int e = 0; e < 8; ++e) {
@@ -1181,7 +1168,7 @@ __global__ void __launch_bounds__(kThreadsTC, 1) v5tc_frontend_kernel(const V5St
                     const int c0 = t * 32 + i0;
                     float m[8], cr[8];
                     tmem_ld8(lane_addr + kColMain + c0, m);
-                    tmem_ld8_corr(lane_addr + kColCorr + c0, cr);
+                    tmem_ld8(lane_addr + kColCorr + c0, cr);
                     tmem_wait_ld();
 #pragma unroll
                     for (int e = 0; e < 8; ++e) {
@@ -1263,7 +1250,7 @@ __global__ void __launch_bounds__(kThreadsTC, 1) v5tc_frontend_kernel(const V5St
                     const int c0 = t * 32 + i0;
                     float m[8], cr[8];
                     tmem_ld8(lane_addr + kColMain + c0, m);
-                    tmem_ld8_corr(lane_addr + kColCorr + c0, cr);
+                    tmem_ld8(lane_addr + kColCorr + c0, cr);
                     tmem_wait_ld();
 #pragma unroll
                     for (int e = 0; e < 8; ++e) {
@@ -1329,7 +1316,7 @@ __global__ void __launch_bounds__(kThreadsTC, 1) v5tc_frontend_kernel(const V5St
                 const int c0 = cg * 8;
                 float m[8], cr[8], v[8];
                 tmem_ld8(lane_addr + kColMain + c0, m);
-                tmem_ld8_corr(lane_addr + kColCorr + c0, cr);
+                tmem_ld8(lane_addr + kColCorr + c0, cr);
                 tmem_wait_ld();
                 float si[8];
                 inv_scales8(amax + 3 * kTile + c0, iw, si);
@@ -1387,7 +1374,7 @@ __global__ void __launch_bounds__(kThreadsTC, 1) v5tc_frontend_kernel(const V5St
                 const int c0 = cg * 8;
                 float m[8], cr[8], v[8];
                 tmem_ld8(lane_addr + kColMain + c0, m);
-                tmem_ld8_corr(lane_addr + kColCorr + c0, cr);
+                tmem_ld8(lane_addr + kColCorr + c0, cr);
                 tmem_wait_ld();
                 float si[8];
                 inv_scales8(amax + 4 * kTile + c0, iw, si);

@@ -93,8 +93,8 @@ class StreamEngine:
 
     # ------------------------------------------------------------------ plumbing
     def set_math(self, math: str) -> None:
-        """'fp32' = packed FP32 FMA kernels; 'tc' = tcgen05 tensor cores with the 3-way BF16 split; 'tc16' (v5) = one-frame
-        steps with the 2-way FP16 split and per-stream scaling (3 products per MAC), other steps as 'tc'; 'fft' (v4, its
+        """'fp32' = packed FP32 FMA kernels; 'tc' = tcgen05 tensor cores with the 3-way BF16 split; 'tc16' (v5, its
+        default) = tensor cores with the 2-way FP16 split and per-stream scaling (3 products per MAC); 'fft' (v4, its
         default) = the STFT as a double-precision FFT plus a tensor-core correction for the basis' float32 rounding."""
         code = {"fp32": capi.MATH_FP32, "tc": capi.MATH_TC, "tc16": capi.MATH_TC16, "fft": capi.MATH_FFT}.get(math)
         if code is None:
