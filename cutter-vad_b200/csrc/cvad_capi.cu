@@ -5,6 +5,7 @@
 // pinned staging used by the host-buffer entry point.  There is no CPU fallback: if no
 // sm_100 device is present every compute entry point fails with CVAD_E_NOGPU.
 #include <algorithm>
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -91,7 +92,8 @@ struct cvad_engine {
     DevBuf d_mono;                     // interleaved multi-channel input averaged to mono (cvad_step_args::channels > 1)
     DevBuf d_res;                      // resampled 16 kHz audio of the step being launched
     DevBuf d_rate_lists;               // mixed-rate steps: [4][n] stream lists + 4 counters
-    DevBuf d_state_blk, h_state_blk;   // cvad_get_state: one slot's packed state (device scratch, pinned host)
+    DevBuf d_state_blk, h_state_blk;   // cvad_get_state / cvad_export_states / cvad_import_states: records (device scratch, pinned host)
+    uint64_t fingerprint = 0;          // cvad_model_fingerprint
     // host-buffer steps run on kLanes lanes so that later steps' H2D copies overlap earlier steps' kernels and D2H
     struct Lane {
         cudaStream_t stream = nullptr;
@@ -1321,6 +1323,17 @@ int cvad_create(const float *weights, size_t n_weight_floats, int model_version,
     e->v4_t2 = v4_8k;
     e->max_streams = max_streams;
     e->num_sms = pr.multiProcessorCount;
+    {
+        // cvad_model_fingerprint: FNV-1a 64 over the model version (little-endian int32) and the weight blob's bytes
+        const int32_t mv = v4_8k ? CVAD_MODEL_V4_8K : model_version;
+        uint64_t hsh = 0xcbf29ce484222325ull;
+        auto mix = [&hsh](const unsigned char *p, size_t n) {
+            for (size_t i = 0; i < n; ++i) { hsh ^= p[i]; hsh *= 0x100000001b3ull; }
+        };
+        mix(reinterpret_cast<const unsigned char *>(&mv), sizeof(mv));
+        mix(reinterpret_cast<const unsigned char *>(weights), n_weight_floats * sizeof(float));
+        e->fingerprint = hsh;
+    }
     auto bail = [&](int rc) {
         g_create_error = e->err;
         cvad_destroy(e);
@@ -1608,46 +1621,35 @@ int cvad_configure(cvad_engine *e, int n, const int32_t *slots, double vad_start
     return CVAD_OK;
 }
 
-namespace {
-// one slot's state in one block of 1,048 bytes: h[128] c[128] f32 | is_voice_active, start count, end count, 0 | frames_done
-constexpr size_t kStateBlock = 256 * sizeof(float) + 4 * sizeof(int) + sizeof(long long);
-__global__ void pack_state_kernel(const float *h, const float *c, const int *act, const int *sc, const int *ec,
-                                  const long long *fd, int slot, unsigned char *out) {
-    const int t = threadIdx.x;
-    float *f = reinterpret_cast<float *>(out);
-    if (t < 128) f[t] = h[cvad::state_at(t, slot)];
-    else f[t] = c[cvad::state_at(t - 128, slot)];
-    if (t == 0) {
-        int *w = reinterpret_cast<int *>(out + 256 * sizeof(float));
-        w[0] = act[slot]; w[1] = sc[slot]; w[2] = ec[slot]; w[3] = 0;
-        *reinterpret_cast<long long *>(out + 256 * sizeof(float) + 4 * sizeof(int)) = fd[slot];
-    }
-}
-}  // namespace
+}  // extern "C"
 
-// One small kernel packs the slot's words, ONE device-to-host copy brings them over (the per-call path of the drop-in
-// wrapper reads the state after every call: seven separate synchronous copies were 0.1 ms of its 0.4 ms).
+#include "cvad_state.cuh"
+
+extern "C" {
+
+// cvad_get_state is export_states_kernel for one record: one small kernel packs the slot's words, ONE device-to-host copy
+// brings them over (the per-call path of the drop-in wrapper reads the state after every call: seven separate synchronous
+// copies were 0.1 ms of its 0.4 ms).
 int cvad_get_state(cvad_engine *e, int slot, float *h, float *c, int32_t *sm, int64_t *frames_done) {
     if (!e) return CVAD_E_INVALID;
     if (slot < 0 || slot >= e->max_streams) return fail(e, CVAD_E_CAPACITY, "slot id out of range");
     CU_TRY(e, cudaSetDevice(e->device));
     { int rcq = quiesce(e); if (rcq) return rcq; }
-    int rc = grow(e, e->d_state_blk, kStateBlock);
+    const size_t bytes = sizeof(cvad_stream_state);
+    int rc = grow(e, e->d_state_blk, bytes);
     if (rc) return rc;
-    if ((rc = grow_host(e, e->h_state_blk, kStateBlock))) return rc;
-    unsigned char *d = static_cast<unsigned char *>(e->d_state_blk.p), *hb = static_cast<unsigned char *>(e->h_state_blk.p);
-    pack_state_kernel<<<1, 256, 0, e->stream>>>(e->h_state, e->c_state, e->sm_active, e->sm_scount, e->sm_ecount, e->frames_done, slot, d);
+    if ((rc = grow_host(e, e->h_state_blk, bytes))) return rc;
+    export_states_kernel<<<1, 256, 0, e->stream>>>(state_arrays(e), nullptr, slot, 1, static_cast<uint32_t *>(e->d_state_blk.p));
     CU_TRY(e, cudaGetLastError());
-    CU_TRY(e, cudaMemcpyAsync(hb, d, kStateBlock, cudaMemcpyDeviceToHost, e->stream));
+    CU_TRY(e, cudaMemcpyAsync(e->h_state_blk.p, e->d_state_blk.p, bytes, cudaMemcpyDeviceToHost, e->stream));
     CU_TRY(e, cudaStreamSynchronize(e->stream));
-    if (h) std::memcpy(h, hb, 128 * sizeof(float));
-    if (c) std::memcpy(c, hb + 128 * sizeof(float), 128 * sizeof(float));
-    if (sm) std::memcpy(sm, hb + 256 * sizeof(float), 4 * sizeof(int));
-    if (frames_done) {
-        long long v = 0;
-        std::memcpy(&v, hb + 256 * sizeof(float) + 4 * sizeof(int), sizeof(v));
-        *frames_done = v;
+    const cvad_stream_state *r = static_cast<const cvad_stream_state *>(e->h_state_blk.p);
+    if (h) std::memcpy(h, r->h, 128 * sizeof(float));
+    if (c) std::memcpy(c, r->c, 128 * sizeof(float));
+    if (sm) {
+        sm[0] = r->is_voice_active; sm[1] = r->voice_start_frame_count; sm[2] = r->voice_end_frame_count; sm[3] = 0;
     }
+    if (frames_done) *frames_done = r->frames_done;
     return CVAD_OK;
 }
 

@@ -871,3 +871,147 @@ int cvad_feeder_deliver_only(cvad_feeder *f, const float *probs, const uint8_t *
 }
 
 }  // extern "C"
+
+// ---- row snapshots (layout in include/cutter_vad_b200.h, above cvad_feeder_export)
+namespace {
+
+struct SnapHeader {
+    uint32_t magic, version;
+    int32_t pcm_format, frame_len, hop, src_rate, n, zero;
+};
+struct SnapRow {
+    int32_t rate, n_in, payload, denoise;
+    double start_p;
+    int32_t active, zero;
+    int64_t skip, n_pending, n_pre_roll, n_segment;
+};
+static_assert(sizeof(SnapHeader) == 32 && sizeof(SnapRow) == 64, "feeder snapshot layout");
+
+// range and distinctness of a slot list (mark / mark_gen as in push_many; caller holds the lock)
+int feeder_check_slots(cvad_feeder *f, int n, const int32_t *slots) {
+    if (n < 0 || (n > 0 && !slots)) return ffail(f, CVAD_E_INVALID, "bad slot list");
+    if (++f->mark_gen == 0u) { std::fill(f->mark.begin(), f->mark.end(), 0u); f->mark_gen = 1u; }
+    for (int i = 0; i < n; ++i) {
+        if (slots[i] < 0 || slots[i] >= f->max_streams) return ffail(f, CVAD_E_CAPACITY, "slot id out of range");
+        if (f->mark[slots[i]] == f->mark_gen) return ffail(f, CVAD_E_INVALID, "slot " + std::to_string(slots[i]) + " is listed twice");
+        f->mark[slots[i]] = f->mark_gen;
+    }
+    return CVAD_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int cvad_feeder_export(cvad_feeder *f, int n, const int32_t *slots, void *out, size_t out_bytes, size_t *needed) {
+    if (!f) return CVAD_E_INVALID;
+    std::lock_guard<std::mutex> lk(f->mu);
+    if (const int rc = feeder_check_slots(f, n, slots)) return rc;
+    size_t total = sizeof(SnapHeader);
+    for (int i = 0; i < n; ++i) {
+        const int s = slots[i];
+        if (!f->opn[s]) return ffail(f, CVAD_E_INVALID, "export: stream " + std::to_string(s) + " is not open");
+        total += sizeof(SnapRow) + (size_t)f->fill[s] * f->es +
+                 (f->slot[s].pre_roll.size() + f->slot[s].segment.size()) * sizeof(float);
+    }
+    if (needed) *needed = total;
+    if (!out) return CVAD_OK;
+    if (out_bytes < total) return ffail(f, CVAD_E_CAPACITY, "export: out_bytes < needed");
+    unsigned char *p = static_cast<unsigned char *>(out);
+    const SnapHeader hd{CVAD_FEEDER_SNAPSHOT_MAGIC, CVAD_FEEDER_SNAPSHOT_VERSION, f->pcm_format, f->frame_len, f->hop,
+                        f->src_rate, n, 0};
+    std::memcpy(p, &hd, sizeof(hd));
+    p += sizeof(hd);
+    for (int i = 0; i < n; ++i) {
+        const int s = slots[i];
+        const cvad_feeder::Slot &sl = f->slot[s];
+        const SnapRow r{sl.rate, sl.n_in, f->pay[s], sl.denoise ? 1 : 0, sl.start_p, f->act[s] ? 1 : 0, 0, f->skp[s],
+                        f->fill[s], (int64_t)sl.pre_roll.size(), (int64_t)sl.segment.size()};
+        std::memcpy(p, &r, sizeof(r));
+        p += sizeof(r);
+        const size_t pb = (size_t)f->fill[s] * f->es;
+        if (pb) std::memcpy(p, f->arena + (size_t)s * f->cap * f->es, pb);
+        p += pb;
+        if (!sl.pre_roll.empty()) std::memcpy(p, sl.pre_roll.data(), sl.pre_roll.size() * sizeof(float));
+        p += sl.pre_roll.size() * sizeof(float);
+        if (!sl.segment.empty()) std::memcpy(p, sl.segment.data(), sl.segment.size() * sizeof(float));
+        p += sl.segment.size() * sizeof(float);
+    }
+    return CVAD_OK;
+}
+
+int cvad_feeder_import(cvad_feeder *f, int n, const int32_t *slots, const void *in, size_t in_bytes) {
+    if (!f) return CVAD_E_INVALID;
+    if (!in) return ffail(f, CVAD_E_INVALID, "import: blob is NULL");
+    std::lock_guard<std::mutex> lk(f->mu);
+    if (const int rc = feeder_check_slots(f, n, slots)) return rc;
+    // the whole blob is checked before any slot changes
+    const unsigned char *b = static_cast<const unsigned char *>(in);
+    SnapHeader hd{};
+    if (in_bytes < sizeof(hd)) return ffail(f, CVAD_E_INVALID, "import: blob shorter than its header");
+    std::memcpy(&hd, b, sizeof(hd));
+    if (hd.magic != CVAD_FEEDER_SNAPSHOT_MAGIC) return ffail(f, CVAD_E_INVALID, "import: not a feeder snapshot (bad magic)");
+    if (hd.version != CVAD_FEEDER_SNAPSHOT_VERSION)
+        return ffail(f, CVAD_E_INVALID, "import: feeder snapshot version " + std::to_string(hd.version) + " is not supported");
+    if (hd.pcm_format != f->pcm_format) return ffail(f, CVAD_E_INVALID, "import: the blob's PCM format differs from this feeder's");
+    if (hd.src_rate != f->src_rate || hd.frame_len != f->frame_len || hd.hop != f->hop)
+        return ffail(f, CVAD_E_INVALID, "import: the blob's framing (frame_len, hop, source rate) differs from this feeder's");
+    if (hd.n != n) return ffail(f, CVAD_E_INVALID, "import: the blob holds " + std::to_string(hd.n) + " rows, not n");
+    std::vector<size_t> at((size_t)n);
+    size_t pos = sizeof(hd);
+    int64_t longest = 0;
+    for (int i = 0; i < n; ++i) {
+        SnapRow r{};
+        if (in_bytes - pos < sizeof(r)) return ffail(f, CVAD_E_INVALID, "import: blob truncated at row " + std::to_string(i));
+        std::memcpy(&r, b + pos, sizeof(r));
+        at[(size_t)i] = pos;
+        const std::string row = "import: row " + std::to_string(i) + ": ";
+        const int want_rate = f->src_rate ? f->src_rate : r.rate;
+        if (r.rate != want_rate || (r.rate != 16000 && rate_index(r.rate) < 0))
+            return ffail(f, CVAD_E_INVALID, row + "source rate " + std::to_string(r.rate) + " does not fit this feeder");
+        if (r.n_in != rate_n_in(r.rate)) return ffail(f, CVAD_E_INVALID, row + "n_in does not match its rate");
+        if (r.payload < CVAD_PAYLOAD_NONE || r.payload > CVAD_PAYLOAD_FRAMES) return ffail(f, CVAD_E_INVALID, row + "unknown payload mode");
+        if ((r.denoise != 0 && r.denoise != 1) || (r.active != 0 && r.active != 1) || !(r.start_p >= 0.0 && r.start_p <= 1.0))
+            return ffail(f, CVAD_E_INVALID, row + "bad denoise / active flag or start probability");
+        if (r.skip < 0 || r.n_pending < 0 || r.n_pre_roll < 0 || r.n_segment < 0)
+            return ffail(f, CVAD_E_INVALID, row + "negative length");
+        pos += sizeof(r);
+        const uint64_t tail = (uint64_t)r.n_pending * f->es + ((uint64_t)r.n_pre_roll + (uint64_t)r.n_segment) * sizeof(float);
+        if ((uint64_t)(in_bytes - pos) < tail || r.n_pending > (int64_t)(in_bytes / f->es) ||
+            r.n_pre_roll > (int64_t)in_bytes || r.n_segment > (int64_t)in_bytes)
+            return ffail(f, CVAD_E_INVALID, row + "blob truncated");
+        pos += (size_t)tail;
+        longest = std::max(longest, r.n_pending);
+    }
+    if (pos != in_bytes) return ffail(f, CVAD_E_INVALID, "import: " + std::to_string(in_bytes - pos) + " bytes after the last row");
+    if (const int rc = feeder_grow_arena(f, longest)) return rc;
+    for (int i = 0; i < n; ++i) {
+        SnapRow r{};
+        std::memcpy(&r, b + at[(size_t)i], sizeof(r));
+        const unsigned char *p = b + at[(size_t)i] + sizeof(r);
+        const int s = slots[i];
+        cvad_feeder::Slot &sl = f->slot[s];
+        f->opn[s] = 1;
+        f->pay[s] = (uint8_t)r.payload;
+        f->act[s] = (uint8_t)r.active;
+        f->skp[s] = r.skip;
+        sl.rate = r.rate;
+        sl.n_in = r.n_in;
+        sl.denoise = r.denoise != 0;
+        sl.start_p = r.start_p;
+        const size_t pb = (size_t)r.n_pending * f->es;
+        if (pb) std::memcpy(f->arena + (size_t)s * f->cap * f->es, p, pb);
+        f->fill[s] = r.n_pending;
+        p += pb;
+        // a row that carries no audio keeps none (its payload mode may have been lowered since the export)
+        const bool audio = r.payload >= CVAD_PAYLOAD_SEGMENTS;
+        sl.pre_roll.resize(audio ? (size_t)r.n_pre_roll : 0);
+        if (!sl.pre_roll.empty()) std::memcpy(sl.pre_roll.data(), p, sl.pre_roll.size() * sizeof(float));
+        p += (size_t)r.n_pre_roll * sizeof(float);
+        sl.segment.resize(audio ? (size_t)r.n_segment : 0);
+        if (!sl.segment.empty()) std::memcpy(sl.segment.data(), p, sl.segment.size() * sizeof(float));
+    }
+    return CVAD_OK;
+}
+
+}  // extern "C"

@@ -9,6 +9,7 @@ The Silero arithmetic runs in hand-written sm_100a CUDA kernels behind the C ABI
 from .core.async_vad_wrapper import AsyncVADWrapper
 from .core.batched_manager import BatchedVADManager, StreamEvent
 from .core.sharded_manager import ShardedVADManager
+from .core.stream_snapshot import StreamSnapshot
 from .core.config import SampleRate, SileroModelVersion, VADConfig
 from .core.exceptions import ConfigurationError, ModelNotFoundError, VADError
 from .core.vad_wrapper import VADWrapper
@@ -17,6 +18,6 @@ from .utils.wav_writer import WAVWriter
 
 __version__ = "1.0.0+b200"
 
-__all__ = ["VADWrapper", "AsyncVADWrapper", "BatchedVADManager", "ShardedVADManager", "StreamEvent", "VADConfig", "SampleRate",
+__all__ = ["VADWrapper", "AsyncVADWrapper", "BatchedVADManager", "ShardedVADManager", "StreamEvent", "StreamSnapshot", "VADConfig", "SampleRate",
            "SileroModelVersion", "VADError", "ModelNotFoundError", "ConfigurationError", "AudioUtils",
            "WAVWriter", "__version__"]

@@ -34,11 +34,12 @@ from typing import Callable, Dict, List, NamedTuple, Optional, Sequence
 import numpy as np
 
 from ..engine import capi
-from ..engine.feeder import FeederError, StreamFeeder
-from ..engine.stream_engine import StreamEngine
+from ..engine.feeder import FeederError, StreamFeeder, set_row_payloads
+from ..engine.stream_engine import EngineError, StreamEngine
 from ..utils.wav_writer import WAVWriter
 from .config import SileroModelVersion, VADConfig
 from .exceptions import AudioProcessingError, CallbackError, ConfigurationError, VADError
+from .stream_snapshot import SnapshotStream, StreamSnapshot
 
 
 class StreamEvent(NamedTuple):
@@ -120,6 +121,7 @@ class BatchedVADManager:
         except Exception as exc:
             raise VADError(f"Failed to initialize VAD processor: {exc}")
         self.max_streams = max_streams
+        self.model_version = model_version.value
         self._free = list(range(max_streams - 1, -1, -1))
         self._streams: Dict[int, _Stream] = {}
         self._lock = threading.Lock()
@@ -356,6 +358,110 @@ class BatchedVADManager:
             cb(*args)
         except Exception as exc:
             raise CallbackError(name, exc)
+
+    # ------------------------------------------------------------------ stream snapshots
+    def snapshot_streams(self, stream_ids: Optional[Sequence[int]] = None) -> StreamSnapshot:
+        """Freeze open streams (all of them by default) between steps: the engine's records and the feeder's rows are
+        taken under the manager lock, so they describe the same instant.  The streams keep running here; audio pushed
+        after the snapshot belongs to them only.  A move is snapshot, close_stream, then restore_streams elsewhere."""
+        with self._lock:
+            ids = sorted(self._streams) if stream_ids is None else [int(s) for s in stream_ids]
+            for s in ids:
+                self._stream(s)
+            if len(set(ids)) != len(ids):
+                raise VADError("snapshot_streams: a stream is listed twice")
+            try:
+                states = self._engine.export_states(ids) if ids else np.zeros(0, capi.STATE_DTYPE)
+                rows = self._feeder.export_rows(ids)
+            except (EngineError, FeederError) as exc:
+                raise VADError(f"snapshot_streams failed: {exc.message}")
+            streams = []
+            for s in ids:
+                st = self._streams[s]
+                streams.append(SnapshotStream(s, st.config._to_serializable_dict(), self._payload_mode(st), st.active,
+                                              [f.copy() for f in st.pre_roll], [f.copy() for f in st.segment]))
+            return StreamSnapshot(self.model_version, self._engine.fingerprint, int(self.pcm_format), self.frame_len,
+                                  self.hop, None if self.mixed else self.source_rate, streams, states, rows)
+
+    def restore_streams(self, snapshot: StreamSnapshot,
+                        callbacks: Optional[Dict[int, Dict[str, Callable]]] = None) -> Dict[int, int]:
+        """Open the snapshot's streams here, each continuing exactly where it was: same LSTM state, state machine,
+        frame count (event frame indices continue), pending samples, pre-roll and half-built segment.  `callbacks` maps
+        a stream's id in the snapshot to dict(on_voice_start=..., on_voice_end=..., on_voice_continue=...).  All or
+        nothing; -> {id in the snapshot: id here}.
+
+        ConfigurationError, with nothing opened: another model version or weights (fingerprint), PCM format, framing or
+        source-rate mode; fewer free slots than streams; or a stream in the middle of voice (active, or with a pre-roll)
+        whose new callbacks want audio its snapshot did not carry (it was taken with callbacks that wanted less).
+        The math mode may differ: the state is FP32 in every mode."""
+        snap = snapshot
+        callbacks = callbacks or {}
+        if snap.model_version != self.model_version:
+            raise ConfigurationError("model_version", snap.model_version, f"this manager runs {self.model_version}")
+        if int(snap.fingerprint) != self._engine.fingerprint:
+            raise ConfigurationError("fingerprint", f"{int(snap.fingerprint):016x}",
+                                     "the snapshot was taken with other model weights")
+        if int(snap.pcm_format) != int(self.pcm_format):
+            raise ConfigurationError("pcm_format", str(snap.pcm_format), f"this manager takes pcm_format {self.pcm_format}")
+        if (snap.frame_len, snap.hop) != (self.frame_len, self.hop):
+            raise ConfigurationError("frame_len/hop", f"{snap.frame_len}/{snap.hop}",
+                                     f"this manager frames {self.frame_len}/{self.hop}")
+        if snap.source_rate != (None if self.mixed else self.source_rate):
+            raise ConfigurationError("source_rate", str(snap.source_rate),
+                                     f"this manager takes {'mixed-rate' if self.mixed else self.source_rate} streams")
+        n = len(snap.streams)
+        if len(snap.states) != n:
+            raise VADError("invalid stream snapshot: engine records do not match the stream list")
+        if len(set(snap.stream_ids)) != n:
+            raise VADError("invalid stream snapshot: a stream id appears twice")
+        new_streams: List[_Stream] = []
+        for k, ss in enumerate(snap.streams):
+            try:
+                cfg = VADConfig.from_dict(dict(ss.config))
+            except Exception as exc:
+                raise VADError(f"invalid stream snapshot: stream {ss.stream_id}: bad config ({exc})")
+            cb = callbacks.get(ss.stream_id, {})
+            unknown = set(cb) - {"on_voice_start", "on_voice_end", "on_voice_continue"}
+            if unknown:
+                raise ConfigurationError("callbacks", ", ".join(sorted(unknown)))
+            st = _Stream(config=cfg, writer=WAVWriter(cfg.output_wav_sample_rate, cfg.output_wav_bit_depth, 1),
+                         on_start=cb.get("on_voice_start"), on_end=cb.get("on_voice_end"),
+                         on_continue=cb.get("on_voice_continue"))
+            carried = ss.payload >= capi.PAYLOAD_SEGMENTS
+            # in the middle of voice: active, or in the pre-roll -- frames at or above the start threshold since the
+            # last one below it, which is exactly when the engine's start counter is above 0 (the feeder's pre-roll
+            # follows the same rule, but only streams that carried audio kept one)
+            rec = snap.states[k]
+            mid_voice = bool(rec["is_voice_active"]) or int(rec["voice_start_frame_count"]) > 0 or ss.active or \
+                bool(ss.pre_roll)
+            if st.wants_audio and not carried and mid_voice:
+                raise ConfigurationError("callbacks", f"stream {ss.stream_id}",
+                                         "the stream is in the middle of voice and its snapshot carries no audio for "
+                                         "the voice_end / voice_continue callbacks")
+            if st.wants_audio:
+                st.active, st.pre_roll, st.segment = ss.active, list(ss.pre_roll), list(ss.segment)
+            new_streams.append(st)
+        try:
+            rows = set_row_payloads(snap.feeder_rows, [self._payload_mode(st) for st in new_streams])
+        except ValueError as exc:
+            raise VADError(f"invalid stream snapshot: {exc}")
+        with self._lock:
+            if len(self._free) < n:
+                raise ConfigurationError("max_streams", str(self.max_streams),
+                                         f"{n} streams to restore, {len(self._free)} slots free")
+            ids = [self._free.pop() for _ in range(n)]
+            try:
+                if n:
+                    self._engine.import_states(ids, snap.states)
+                self._feeder.import_rows(ids, rows)
+            except (EngineError, FeederError) as exc:
+                self._free.extend(reversed(ids))
+                if n:
+                    self._engine.reset(ids)
+                raise VADError(f"invalid stream snapshot: {exc.message}")
+            for sid, st in zip(ids, new_streams):
+                self._streams[sid] = st
+            return {ss.stream_id: sid for ss, sid in zip(snap.streams, ids)}
 
     # ------------------------------------------------------------------ lock-step block API
     def step_block(self, audio: np.ndarray, stream_ids: Optional[Sequence[int]] = None):

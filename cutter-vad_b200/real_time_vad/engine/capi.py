@@ -10,6 +10,8 @@ import ctypes as C
 import os
 from pathlib import Path
 
+import numpy as np
+
 PKG_ROOT = Path(__file__).resolve().parents[2]          # .../cutter-vad_b200
 LIB_PATH = PKG_ROOT / "libcvad_b200.so"
 DEV_LIB_PATH = PKG_ROOT / "libcvad_b200_dev.so"     # development probes (csrc/cvad_dev.cu): tests and tools only
@@ -32,7 +34,16 @@ EXPORTS = (
     "cvad_feeder_create", "cvad_feeder_destroy", "cvad_feeder_last_error", "cvad_feeder_open", "cvad_feeder_close",
     "cvad_feeder_clear", "cvad_feeder_is_active", "cvad_feeder_pending", "cvad_feeder_push", "cvad_feeder_push_many",
     "cvad_feeder_step", "cvad_feeder_gather_only", "cvad_feeder_deliver_only",
+    "cvad_model_fingerprint", "cvad_export_states", "cvad_import_states", "cvad_feeder_export", "cvad_feeder_import",
 )
+
+# cvad_stream_state: one slot's engine state, 1,072 bytes without padding (cvad_export_states / cvad_import_states)
+STATE_DTYPE = np.dtype([("h", "<f4", (128,)), ("c", "<f4", (128,)), ("frames_done", "<i8"),
+                        ("vad_start_probability", "<f8"), ("vad_end_probability", "<f8"),
+                        ("is_voice_active", "<i4"), ("voice_start_frame_count", "<i4"), ("voice_end_frame_count", "<i4"),
+                        ("n_start", "<i4"), ("n_end", "<i4"), ("enable_denoising", "<i4")])
+assert STATE_DTYPE.itemsize == 1072
+FEEDER_SNAPSHOT_MAGIC, FEEDER_SNAPSHOT_VERSION = 0x53465643, 1
 
 
 class Event(C.Structure):
@@ -165,5 +176,10 @@ def lib() -> C.CDLL:
     L.cvad_feeder_step.argtypes = [vp, C.POINTER(FeederResult)]
     L.cvad_feeder_gather_only.argtypes = [vp, C.POINTER(FeederResult)]
     L.cvad_feeder_deliver_only.argtypes = [vp, vp, vp, C.POINTER(FeederResult)]
+    L.cvad_model_fingerprint.argtypes = [vp, C.POINTER(C.c_uint64)]
+    L.cvad_export_states.argtypes = [vp, i32, vp, vp]
+    L.cvad_import_states.argtypes = [vp, i32, vp, vp]
+    L.cvad_feeder_export.argtypes = [vp, i32, vp, vp, C.c_size_t, C.POINTER(C.c_size_t)]
+    L.cvad_feeder_import.argtypes = [vp, i32, vp, vp, C.c_size_t]
     _lib = L
     return L

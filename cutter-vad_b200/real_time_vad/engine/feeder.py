@@ -9,6 +9,7 @@ all in native code, so that Python only sees the frames something happened on.
 from __future__ import annotations
 
 import ctypes as C
+import struct
 from typing import List, NamedTuple, Optional, Sequence
 
 import numpy as np
@@ -58,6 +59,25 @@ _DELIV_DT = np.dtype([("slot", "<i4"), ("stream", "<i4"), ("step_frame", "<i4"),
                       ("segment", "<u8"), ("segment_len", "<i8"), ("frame_len", "<i4"), ("prob", "<f4"),
                       ("raw", "<u8"), ("raw_len", "<i8")])
 assert _EVENT_DT.itemsize == C.sizeof(capi.Event) and _DELIV_DT.itemsize == C.sizeof(capi.Delivery)
+
+
+def set_row_payloads(blob: bytes, payloads: Sequence[int]) -> bytes:
+    """A copy of an export_rows blob with row i's payload mode set to payloads[i] (CVAD_PAYLOAD_*): the payload mode
+    follows the callbacks a restored stream gets, not the ones it had.  Raises ValueError for a malformed blob."""
+    b = bytearray(blob)
+    try:
+        magic, version, pcm, _fl, _hop, _sr, n, _z = struct.unpack_from("<IIiiiiii", b, 0)
+        if magic != capi.FEEDER_SNAPSHOT_MAGIC or version != capi.FEEDER_SNAPSHOT_VERSION or n != len(payloads):
+            raise ValueError("not a feeder snapshot with one row per stream")
+        es = 4 if pcm == capi.PCM_F32 else 2
+        pos = 32
+        for i in range(n):
+            struct.pack_into("<i", b, pos + 8, int(payloads[i]))
+            n_pending, n_pre, n_seg = struct.unpack_from("<qqq", b, pos + 40)
+            pos += 64 + n_pending * es + (n_pre + n_seg) * 4
+    except struct.error as exc:
+        raise ValueError(f"truncated feeder snapshot: {exc}")
+    return bytes(b)
 
 
 def _view(ptr: int, dtype, count: int) -> np.ndarray:
@@ -122,6 +142,29 @@ class StreamFeeder:
 
     def pending(self, slot: int) -> int:
         return int(self._check(self._L.cvad_feeder_pending(self._h, int(slot))))
+
+    # ------------------------------------------------------------------ row snapshots
+    def export_rows(self, slots: Sequence[int]) -> bytes:
+        """Pending samples, pre-roll and half-built segment of open `slots` as one persistable blob (cvad_feeder_export;
+        layout in include/cutter_vad_b200.h)."""
+        ids = np.ascontiguousarray(slots, dtype=np.int32)
+        need = C.c_size_t(0)
+        self._check(self._L.cvad_feeder_export(self._h, int(ids.size), ids.ctypes.data, None, 0, C.byref(need)))
+        while True:
+            # pushes from other threads may grow the rows between sizing and copying: the call then reports the new
+            # size (CVAD_E_CAPACITY, nothing written) and is repeated with room to spare
+            cap = int(need.value) + int(need.value) // 8 + 4096
+            buf = C.create_string_buffer(cap)
+            rc = self._L.cvad_feeder_export(self._h, int(ids.size), ids.ctypes.data, buf, cap, C.byref(need))
+            if rc != capi.E_CAPACITY or int(need.value) <= cap:
+                self._check(rc)
+                return buf.raw[:int(need.value)]
+
+    def import_rows(self, slots: Sequence[int], blob: bytes) -> None:
+        """(Re)open `slots` with the rows of an export_rows blob, in order; the whole blob is checked first."""
+        ids = np.ascontiguousarray(slots, dtype=np.int32)
+        blob = bytes(blob)
+        self._check(self._L.cvad_feeder_import(self._h, int(ids.size), ids.ctypes.data, blob, len(blob)))
 
     # ------------------------------------------------------------------ data path
     def push(self, slot: int, samples: np.ndarray) -> None:

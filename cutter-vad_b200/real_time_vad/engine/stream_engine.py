@@ -203,6 +203,48 @@ class StreamEngine:
         sm = None if sm is None else np.ascontiguousarray(sm, np.int32)
         self._check(self._L.cvad_set_state(self._h, int(slot), _ptr(h), _ptr(c), _ptr(sm)))
 
+    # ------------------------------------------------------------------ stream snapshots
+    @property
+    def fingerprint(self) -> int:
+        """Model version + FNV-1a 64 of the weight blob (cvad_model_fingerprint): records move between engines with
+        equal fingerprints."""
+        v = C.c_uint64(0)
+        self._check(self._L.cvad_model_fingerprint(self._h, C.byref(v)))
+        return int(v.value)
+
+    def export_states(self, slots: Optional[Sequence[int]], device_ptr: Optional[int] = None) -> Optional[np.ndarray]:
+        """The state of `slots` (None = 0..max_streams-1) as capi.STATE_DTYPE records, one per slot in order.  With
+        `device_ptr` the records are written to that device address (len(slots) * 1072 bytes on the engine's device)
+        and None is returned."""
+        n, arr = self._slots(slots)
+        if slots is None:
+            n = self.max_streams
+        if device_ptr is not None:
+            self._check(self._L.cvad_export_states(self._h, n, _ptr(arr), C.c_void_p(int(device_ptr))))
+            return None
+        out = np.zeros(n, capi.STATE_DTYPE)
+        self._check(self._L.cvad_export_states(self._h, n, _ptr(arr), _ptr(out)))
+        return out
+
+    def import_states(self, slots: Optional[Sequence[int]], records) -> None:
+        """Write records into `slots` (None = 0..n-1), all or nothing.  `records`: a STATE_DTYPE array (or bytes of
+        one), or an int device address of len(slots) records on the engine's device."""
+        n, arr = self._slots(slots)
+        if isinstance(records, int):
+            if slots is None:
+                raise EngineError(capi.E_INVALID, "import_states from a device address needs the slot list")
+            self._check(self._L.cvad_import_states(self._h, n, _ptr(arr), C.c_void_p(records)))
+            return
+        rec = np.frombuffer(records, capi.STATE_DTYPE) if isinstance(records, (bytes, bytearray, memoryview)) \
+            else np.ascontiguousarray(records)
+        if rec.dtype != capi.STATE_DTYPE:
+            raise EngineError(capi.E_INVALID, "records must have capi.STATE_DTYPE")
+        if slots is None:
+            n = rec.size
+        elif rec.size != n:
+            raise EngineError(capi.E_INVALID, "len(records) != len(slots)")
+        self._check(self._L.cvad_import_states(self._h, n, _ptr(arr), _ptr(rec)))
+
     # ------------------------------------------------------------------ the hot call
     def _args(self, audio: np.ndarray, slots, n_frames, max_frames, frame_len, hop, pcm_format, src_rate=16000,
               src_rates=None):

@@ -24,6 +24,8 @@
  *   cvad_reset           <- VADProcessor.reset / SileroVADModel.reset     silero_model.py:951-968, :539-546
  *   cvad_get_state/set   <- SileroVADModel.model_state (numpy h/c)        silero_model.py:264-267, :526-537
  *   cvad_last_error      <- the VADError family's messages                src/real_time_vad/core/exceptions.py
+ *   cvad_export/import_states, cvad_feeder_export/import: stream snapshots, which the reference has no equivalent of
+ *                           (its state lives in per-client Python objects, silero_model.py:264-267, :596-628)
  *
  * Plain pointers and sizes only; no torch / numpy types.  All functions return 0
  * on success and a negative CVAD_E_* code on failure (cvad_last_error gives text).
@@ -192,6 +194,37 @@ int cvad_get_state(cvad_engine *e, int slot, float *h, float *c, int32_t *sm, in
 int cvad_set_state(cvad_engine *e, int slot, const float *h, const float *c, const int32_t *sm);
 
 /*
+ * Stream snapshots: everything the engine keeps for one slot, as one fixed-layout record of 1,072 bytes without padding,
+ * so that live streams can move between engines, processes and GPUs (restart a service without dropping its streams).
+ */
+typedef struct cvad_stream_state {
+    float   h[128];                 /* v5: h; v4 / v4_8k: layer 0 then layer 1 (cvad_get_state's order) */
+    float   c[128];
+    int64_t frames_done;            /* frames run since the slot's last reset (cvad_event::stream_frame continues from it) */
+    double  vad_start_probability, vad_end_probability;
+    int32_t is_voice_active, voice_start_frame_count, voice_end_frame_count;
+    int32_t n_start, n_end;         /* configured voice_start/end_frame_count */
+    int32_t enable_denoising;
+} cvad_stream_state;
+
+/* The model version given to cvad_create, then the FNV-1a 64 hash of its weight blob: FNV-1a over the version as a
+   little-endian int32 followed by the blob's bytes.  Records move between engines with equal fingerprints only.  The
+   math mode is not part of it: the state is FP32 in every mode. */
+int cvad_model_fingerprint(const cvad_engine *e, uint64_t *out);
+/* Copy the state of n slots (slots: host memory, distinct ids; NULL = 0..n-1) into out[n] / from in[n].  out / in may be
+   host memory (pageable or pinned) or device memory on the engine's device, 8-byte aligned (CVAD_E_INVALID otherwise);
+   one copy each way.  Device records are read and written on the engine's stream: whatever the caller wrote into them
+   on another stream must be complete before cvad_import_states, and exported records are complete when it returns.
+   Both wait for the steps
+   in flight first and synchronise before returning, like cvad_reset, so the next step (chained device steps included)
+   reads the imported state.  Import is all or nothing: every record is checked on the device first (h and c finite,
+   is_voice_active and enable_denoising 0 or 1, counts and frames_done >= 0, probabilities in [0, 1], n_start and
+   n_end >= 1); one bad record fails the call with CVAD_E_INVALID, cvad_last_error names its index, and no slot changes.
+   CVAD_E_CAPACITY: a slot id out of range; CVAD_E_INVALID: a slot listed twice. */
+int cvad_export_states(cvad_engine *e, int n, const int32_t *slots, cvad_stream_state *out);
+int cvad_import_states(cvad_engine *e, int n, const int32_t *slots, const cvad_stream_state *in);
+
+/*
  * One batched step with HOST buffers: pinned staging + H2D, kernels, D2H, sync.
  * This is what the reference-facing Python mirror calls.
  */
@@ -346,6 +379,30 @@ int cvad_feeder_step(cvad_feeder *f, cvad_feeder_result *out);
    caller-supplied probs / flags [n_streams][max_frames]. */
 int cvad_feeder_gather_only(cvad_feeder *f, cvad_feeder_result *out);
 int cvad_feeder_deliver_only(cvad_feeder *f, const float *probs, const uint8_t *flags, cvad_feeder_result *out);
+
+/*
+ * Row snapshots: the host half of a stream (pending samples, the pre-roll and the half-built segment) as a persistable
+ * blob, the companion of cvad_export_states.  Both calls take the feeder's lock, so a snapshot is a consistent cut
+ * against concurrent pushes.  Export fails with CVAD_E_INVALID for a slot that is not open; out == NULL only reports
+ * *needed, and out_bytes < *needed is CVAD_E_CAPACITY (with *needed set and nothing written).  Import (re)opens the target slots like cvad_feeder_open, after
+ * checking the whole blob (magic, version, the feeder's PCM format and framing -- or, on a mixed-rate feeder, per-slot
+ * rates of 8000 / 16000 / 24000 / 48000 --, payload modes, lengths against in_bytes); a refused blob changes no slot.
+ * A row whose payload mode carries no audio (below CVAD_PAYLOAD_SEGMENTS) is imported without its pre-roll and segment.
+ * Rows grow as cvad_feeder_push makes them grow.  Both work on a feeder built with e == NULL.
+ *
+ * Blob layout, little-endian, no padding:
+ *   header (32 bytes): uint32 magic CVAD_FEEDER_SNAPSHOT_MAGIC, uint32 version CVAD_FEEDER_SNAPSHOT_VERSION,
+ *                      int32 pcm_format, frame_len, hop, src_rate (0 = mixed), int32 n (rows that follow), int32 0
+ *   n rows, in the order of `slots`, each a 64-byte head
+ *       int32 rate, n_in (source samples per model frame), payload (CVAD_PAYLOAD_*), enable_denoising (0 / 1),
+ *       float64 vad_start_probability, int32 voice active (the host mirror, 0 / 1), int32 0,
+ *       int64 skip (hop > frame_len: samples still to drop from the next push), int64 n_pending, n_pre_roll, n_segment
+ *   followed by n_pending samples in the feeder's PCM format, then n_pre_roll and n_segment float32 samples.
+ */
+#define CVAD_FEEDER_SNAPSHOT_MAGIC 0x53465643u   /* "CVFS" */
+#define CVAD_FEEDER_SNAPSHOT_VERSION 1
+int cvad_feeder_export(cvad_feeder *f, int n, const int32_t *slots, void *out, size_t out_bytes, size_t *needed);
+int cvad_feeder_import(cvad_feeder *f, int n, const int32_t *slots, const void *in, size_t in_bytes);
 
 #ifdef __cplusplus
 }
