@@ -683,9 +683,11 @@ __global__ void downmix_kernel(const void *audio, int pcm, long long stride, int
     }
 }
 
-// `chain` (cvad_step_device on a fused one-frame step): the caller enqueued no memset; see cvad_engine::d_evctr
+// `chain` (cvad_step_device on a fused one-frame step): the caller enqueued no memset; see cvad_engine::d_evctr.
+// `input_out` != nullptr (cvad_debug_input): run the input stages only, their output buffer filled with NaN first, and
+// return the device address of the mono 16 kHz samples the model kernels would read in *input_out.
 int launch_step(cvad_engine *e, const cvad_step_args *a, unsigned int *d_status, int commit, float *d_dbg,
-                cudaStream_t stream, unsigned rates_mask = 0xFu, bool chain = false) {
+                cudaStream_t stream, unsigned rates_mask = 0xFu, bool chain = false, const float **input_out = nullptr) {
     if (a->n_streams == 0 || a->max_frames == 0) return CVAD_OK;
     cvad_step_args a_mono;
     if (a->channels > 1) {
@@ -698,6 +700,7 @@ int launch_step(cvad_engine *e, const cvad_step_args *a, unsigned int *d_status,
                                               : (long long)(a->max_frames - 1) * a->hop + a->frame_len;
         int rcg = grow(e, e->d_mono, (size_t)a->n_streams * (size_t)frames * sizeof(float));
         if (rcg) return rcg;
+        if (input_out) CU_TRY(e, cudaMemsetAsync(e->d_mono.p, 0xFF, (size_t)a->n_streams * (size_t)frames * sizeof(float), stream));
         const long long total = (long long)a->n_streams * frames;
         const int grid = (int)std::min<long long>((total + 255) / 256, (long long)e->num_sms * 16);
         downmix_kernel<<<grid, 256, 0, stream>>>(a->audio, a->pcm_format, a->stream_stride, a->channels, a->n_streams, frames,
@@ -719,7 +722,7 @@ int launch_step(cvad_engine *e, const cvad_step_args *a, unsigned int *d_status,
         CU_TRY(e, cudaStreamWaitEvent(stream, e->last_done, 0));
     }
     cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
-    const bool timed = e->timing && !d_dbg;
+    const bool timed = e->timing && !d_dbg && !input_out;
     if (timed) {
         while (e->ev_pool.size() < e->ev_used + 3) {
             cudaEvent_t x;
@@ -746,6 +749,7 @@ int launch_step(cvad_engine *e, const cvad_step_args *a, unsigned int *d_status,
     if (resampled) {
         // stage 0: source-rate chunks -> 16 kHz float frames in HBM; the model kernels then see native input
         if ((rc = grow(e, e->d_res, (size_t)a->n_streams * a->max_frames * 512 * sizeof(float)))) return rc;
+        if (input_out) CU_TRY(e, cudaMemsetAsync(e->d_res.p, 0xFF, (size_t)a->n_streams * a->max_frames * 512 * sizeof(float), stream));
         cvad::ResampleStep r{};
         r.audio = a->audio; r.pcm = a->pcm_format; r.stride = a->stream_stride;
         r.n_streams = a->n_streams; r.n_stiles = n_stiles; r.max_frames = a->max_frames; r.n_frames = a->n_frames;
@@ -844,6 +848,10 @@ int launch_step(cvad_engine *e, const cvad_step_args *a, unsigned int *d_status,
         p.stride = (long long)a->max_frames * 512;
         p.frame_len = 512;
         p.hop = 512;
+    }
+    if (input_out) {
+        *input_out = static_cast<const float *>(p.audio);
+        return CVAD_OK;
     }
     const size_t es = elem_size(p.pcm);
     const uintptr_t addr = reinterpret_cast<uintptr_t>(p.audio);
@@ -1065,20 +1073,38 @@ int quiesce(cvad_engine *e) {
     return CVAD_OK;
 }
 
+// Floats cvad_debug_input writes for the (validated) step `a`: the d_res layout for resampled and mixed-rate steps,
+// the d_mono layout for down-mix-only steps; -1 = the step has no input stage (16 kHz mono).
+long long input_stage_floats(const cvad_step_args *a) {
+    if (a->n_streams == 0 || a->max_frames == 0) return 0;
+    if (a->src_rates || (a->src_rate != 0 && a->src_rate != 16000)) return (long long)a->n_streams * a->max_frames * 512;
+    if (a->channels > 1) return (long long)a->n_streams * ((long long)(a->max_frames - 1) * a->hop + a->frame_len);
+    return -1;
+}
+
 // Enqueue one host-buffer step on `ln` (H2D, kernels, D2H) without waiting for it.
-// `dbg_out` != nullptr turns it into the debug dump (front end only, no commit).
-int step_submit_impl(cvad_engine *e, cvad_engine::Lane &ln, const cvad_step_args *a, float *dbg_out, size_t dbg_floats);
+// `dbg_out` != nullptr turns it into the debug dump (front end only, no commit); `input_out` != nullptr into
+// cvad_debug_input (input stages only, no commit).
+int step_submit_impl(cvad_engine *e, cvad_engine::Lane &ln, const cvad_step_args *a, float *dbg_out, size_t dbg_floats,
+                     float *input_out, size_t input_floats);
 
 // every failure after the lane was marked busy must release it again, whichever statement it comes from
-int step_submit(cvad_engine *e, cvad_engine::Lane &ln, const cvad_step_args *a, float *dbg_out, size_t dbg_floats) {
-    const int rc = step_submit_impl(e, ln, a, dbg_out, dbg_floats);
+int step_submit(cvad_engine *e, cvad_engine::Lane &ln, const cvad_step_args *a, float *dbg_out, size_t dbg_floats,
+                float *input_out = nullptr, size_t input_floats = 0) {
+    const int rc = step_submit_impl(e, ln, a, dbg_out, dbg_floats, input_out, input_floats);
     if (rc != CVAD_OK) ln.busy = false;
     return rc;
 }
 
-int step_submit_impl(cvad_engine *e, cvad_engine::Lane &ln, const cvad_step_args *a, float *dbg_out, size_t dbg_floats) {
+int step_submit_impl(cvad_engine *e, cvad_engine::Lane &ln, const cvad_step_args *a, float *dbg_out, size_t dbg_floats,
+                     float *input_out, size_t input_floats) {
     int rc = validate_args(e, a);
     if (rc) return rc;
+    if (input_out) {
+        const long long nf = input_stage_floats(a);
+        if (nf < 0) return fail(e, CVAD_E_INVALID, "cvad_debug_input: the step has no input stage (16 kHz mono)");
+        if (input_floats < (size_t)nf) return fail(e, CVAD_E_CAPACITY, "cvad_debug_input: out too small");
+    }
     CU_TRY(e, cudaSetDevice(e->device));
     const int n = a->n_streams, T = a->max_frames;
     ln.args = *a;
@@ -1187,6 +1213,14 @@ int step_submit_impl(cvad_engine *e, cvad_engine::Lane &ln, const cvad_step_args
     d.events_out = static_cast<cvad_event *>(ln.d_events.p);
     d.n_events_out = ln.d_nevents;
 
+    if (input_out) {
+        const float *d_in = nullptr;
+        rc = launch_step(e, &d, static_cast<unsigned int *>(ln.d_status.p), 0, nullptr, st, a->src_rates ? rates_mask : 0xFu,
+                         false, &d_in);
+        if (rc) return bail(rc);
+        CU_TRY(e, cudaMemcpyAsync(input_out, d_in, (size_t)input_stage_floats(a) * sizeof(float), cudaMemcpyDeviceToHost, st));
+        return CVAD_OK;
+    }
     float *d_dbg = nullptr;
     if (dbg_out) {
         const size_t nd = e->version == CVAD_MODEL_V4 ? (size_t)cvad::kV4DbgFloats : (size_t)cvad::kDbgFloats;
@@ -1785,6 +1819,21 @@ int cvad_debug_dump(cvad_engine *e, const cvad_step_args *a, float *dbg_out, siz
     rc = step_submit(e, ln, a, dbg_out, dbg_floats);
     if (rc) return rc;
     return step_collect(e, ln, true);
+}
+
+int cvad_debug_input(cvad_engine *e, const cvad_step_args *a, float *out, size_t n_floats) {
+    if (!e) return CVAD_E_INVALID;
+    if (!out) return fail(e, CVAD_E_INVALID, "out is NULL");
+    int rc = quiesce(e);
+    if (rc) return rc;
+    cvad_engine::Lane &ln = e->lanes[0];
+    for (auto &l : e->lanes)
+        if (l.busy) return fail(e, CVAD_E_INVALID, "steps in flight");
+    rc = step_submit(e, ln, a, nullptr, 0, out, n_floats);
+    if (rc) return rc;
+    rc = step_collect(e, ln, true);
+    if (rc < 0) return rc;
+    return (int)input_stage_floats(a);
 }
 
 }  // extern "C"

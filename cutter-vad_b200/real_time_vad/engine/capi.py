@@ -29,6 +29,7 @@ EXPORTS = (
     "cvad_abi_version", "cvad_device_count", "cvad_last_error", "cvad_create", "cvad_destroy",
     "cvad_set_stream", "cvad_reset", "cvad_configure", "cvad_get_state", "cvad_set_state",
     "cvad_step", "cvad_step_submit", "cvad_step_collect", "cvad_step_device", "cvad_sync", "cvad_launch_count", "cvad_debug_dump",
+    "cvad_debug_input",
     "cvad_alloc_pinned", "cvad_free_pinned", "cvad_set_timing", "cvad_read_timing", "cvad_resample_matrix",
     "cvad_set_math", "cvad_get_math", "cvad_set_resampler", "cvad_get_resampler", "cvad_set_profile", "cvad_read_profile", "cvad_read_profile_chain",
     "cvad_feeder_create", "cvad_feeder_destroy", "cvad_feeder_last_error", "cvad_feeder_open", "cvad_feeder_close",
@@ -156,6 +157,7 @@ def lib() -> C.CDLL:
     L.cvad_launch_count.restype = i64
     L.cvad_launch_count.argtypes = [vp]
     L.cvad_debug_dump.argtypes = [vp, C.POINTER(StepArgs), vp, C.c_size_t]
+    L.cvad_debug_input.argtypes = [vp, C.POINTER(StepArgs), vp, C.c_size_t]
     L.cvad_alloc_pinned.restype = vp
     L.cvad_alloc_pinned.argtypes = [C.c_size_t]
     L.cvad_free_pinned.argtypes = [vp]

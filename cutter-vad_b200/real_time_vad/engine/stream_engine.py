@@ -287,15 +287,9 @@ class StreamEngine:
             a.src_rates = sr.ctypes.data
         return a, keep
 
-    def submit(self, audio: np.ndarray, *, slots: Optional[Sequence[int]] = None,
-               n_frames: Optional[Sequence[int]] = None, max_frames: Optional[int] = None,
-               frame_len: int = 512, hop: int = 512, pcm_format: int = capi.PCM_F32,
-               max_events: int = 0, src_rate: int = 16000,
-               src_rates: Optional[Sequence[int]] = None) -> "PendingStep":
-        """Enqueue one step (H2D, kernels, D2H) and return at once; `.collect()` waits for it.
-        Up to four steps may be in flight: later copies overlap earlier steps' kernels and result copies.
-        `audio` must stay untouched until collect (pinned arrays are DMA'd in place)."""
-        audio = np.asarray(audio)
+    @staticmethod
+    def _framing(audio, max_frames, frame_len, hop, src_rate, src_rates):
+        """-> (max_frames, frame_len, hop) of a step over `audio`"""
         if src_rates is not None:
             # per-stream source rates in ONE step: stream i holds max_frames chunks of 512*rate_i/16000 samples
             if max_frames is None:
@@ -306,6 +300,18 @@ class StreamEngine:
             frame_len = hop = src_rate * 512 // 16000
         if max_frames is None:
             max_frames = 0 if audio.shape[1] < frame_len else (audio.shape[1] - frame_len) // hop + 1
+        return max_frames, frame_len, hop
+
+    def submit(self, audio: np.ndarray, *, slots: Optional[Sequence[int]] = None,
+               n_frames: Optional[Sequence[int]] = None, max_frames: Optional[int] = None,
+               frame_len: int = 512, hop: int = 512, pcm_format: int = capi.PCM_F32,
+               max_events: int = 0, src_rate: int = 16000,
+               src_rates: Optional[Sequence[int]] = None) -> "PendingStep":
+        """Enqueue one step (H2D, kernels, D2H) and return at once; `.collect()` waits for it.
+        Up to four steps may be in flight: later copies overlap earlier steps' kernels and result copies.
+        `audio` must stay untouched until collect (pinned arrays are DMA'd in place)."""
+        audio = np.asarray(audio)
+        max_frames, frame_len, hop = self._framing(audio, max_frames, frame_len, hop, src_rate, src_rates)
         a, keep = self._args(audio, slots, n_frames, max_frames, frame_len, hop, pcm_format, src_rate, src_rates)
         n = a.n_streams
         probs = np.empty((n, max_frames), np.float32)
@@ -350,3 +356,20 @@ class StreamEngine:
             res[name] = out[o:o + size].reshape(shape)
             o += size
         return res
+
+    def debug_input(self, audio: np.ndarray, *, src_rate: int = 16000, src_rates: Optional[Sequence[int]] = None,
+                    max_frames: Optional[int] = None, n_frames: Optional[Sequence[int]] = None,
+                    pcm_format: int = capi.PCM_F32, frame_len: int = 512, hop: int = 512) -> np.ndarray:
+        """The float32 mono 16 kHz samples the model kernels would read for the step `submit` would run on the same
+        arguments (cvad_debug_input: input stages only; test hook, engine state untouched).  Resampled and mixed-rate
+        steps -> [n_streams, max_frames * 512], frames beyond a stream's n_frames NaN; down-mix only ->
+        [n_streams, (max_frames - 1) * hop + frame_len]."""
+        audio = np.asarray(audio)
+        max_frames, frame_len, hop = self._framing(audio, max_frames, frame_len, hop, src_rate, src_rates)
+        a, keep = self._args(audio, None, n_frames, max_frames, frame_len, hop, pcm_format, src_rate, src_rates)
+        resampled = src_rates is not None or src_rate not in (0, 16000)
+        per = max_frames * 512 if resampled else max(max_frames - 1, 0) * hop + frame_len
+        out = np.empty((a.n_streams, per if max_frames else 0), np.float32)
+        rc = self._L.cvad_debug_input(self._h, C.byref(a), _ptr(out), out.size)
+        self._check(rc)
+        return out

@@ -283,6 +283,18 @@ int cvad_read_timing(cvad_engine *e, double *frontend_ms, double *recurrent_ms, 
  */
 int cvad_debug_dump(cvad_engine *e, const cvad_step_args *a, float *dbg_out, size_t dbg_floats);
 
+/*
+ * Test hook: run only the input stages of the step `a` describes (the down-mix of interleaved channels and the
+ * resampler, or the pass-through of 16 kHz streams in a mixed-rate step), staged exactly as cvad_step stages it,
+ * and copy to `out` (host) the float32 mono 16 kHz samples the model kernels would read:
+ *   resampled or mixed-rate steps: [n_streams][max_frames * 512];
+ *   down-mix only:                 [n_streams][(max_frames - 1) * hop + frame_len].
+ * The device buffer is filled with 0xFF bytes (NaN) before the stages run, so a frame beyond a stream's n_frames
+ * reads NaN in resampled output.  No model kernel runs and engine state is untouched.  Returns the number of floats
+ * written, CVAD_E_CAPACITY if `n_floats` is too small, CVAD_E_INVALID for a step without an input stage (16 kHz mono).
+ */
+int cvad_debug_input(cvad_engine *e, const cvad_step_args *a, float *out, size_t n_floats);
+
 
 /* ------------------------------------------------------------------------------------------------------------
  * Stream feeder (ABI 3): the host half of the service mode, in native code.
