@@ -544,7 +544,24 @@ int alloc_fill(cvad_engine *e, T **dst, size_t n, T value) {
     return upload(e, dst, tmp);
 }
 
-size_t elem_size(int pcm) { return pcm == CVAD_PCM_F32 ? 4 : 2; }
+bool is_g711(int pcm) { return pcm == CVAD_PCM_ULAW || pcm == CVAD_PCM_ALAW; }
+size_t elem_size(int pcm) { return pcm == CVAD_PCM_F32 ? 4 : is_g711(pcm) ? 1 : 2; }
+
+// ITU-T G.711 expansion of one code to its 16-bit linear value (audioop.ulaw2lin / alaw2lin with width 2): mu-law spans
+// +-32124 (codes 0x7F and 0xFF are 0), A-law +-32256.  Integer arithmetic only, so the decoded sample linear / 32768.0f
+// is exact and equals AudioUtils.pcm_to_float32 of the linear PCM.  The feeder builds its payload tables from it.
+__host__ __device__ inline int g711_linear(int pcm, unsigned code) {
+    if (pcm == CVAD_PCM_ULAW) {
+        const unsigned u = ~code & 0xFFu;
+        const int t = (int)(((u & 0x0Fu) << 3) + 0x84u) << ((u & 0x70u) >> 4);
+        return (u & 0x80u) ? 0x84 - t : t - 0x84;
+    }
+    const unsigned a = (code & 0xFFu) ^ 0x55u;
+    const unsigned seg = (a & 0x70u) >> 4;
+    const int t = (int)((a & 0x0Fu) << 4);
+    const int m = seg == 0 ? t + 8 : (t + 0x108) << (seg - 1);
+    return (a & 0x80u) ? m : -m;
+}
 
 int rate_index(int src_rate) { return src_rate == 8000 ? 0 : src_rate == 24000 ? 1 : src_rate == 48000 ? 2 : -1; }
 int rate_n_in(int src_rate) { return (int)((long long)src_rate * 512 / 16000); }
@@ -555,7 +572,7 @@ int validate_args(cvad_engine *e, const cvad_step_args *a) {
     if (a->n_streams < 0 || a->n_streams > e->max_streams)
         return fail(e, CVAD_E_CAPACITY, "n_streams outside [0, max_streams]");
     if (a->n_streams > 0 && !a->audio) return fail(e, CVAD_E_INVALID, "Audio data is empty");
-    if (a->pcm_format < 0 || a->pcm_format > 2) return fail(e, CVAD_E_INVALID, "unknown pcm_format");
+    if (a->pcm_format < 0 || a->pcm_format > CVAD_PCM_ALAW) return fail(e, CVAD_E_INVALID, "unknown pcm_format");
     if (a->max_frames < 0) return fail(e, CVAD_E_INVALID, "max_frames < 0");
     if (a->max_events < 0) return fail(e, CVAD_E_INVALID, "max_events < 0");
     if (a->channels < 0 || a->channels > 8) return fail(e, CVAD_E_INVALID, "channels outside [0, 8]");
@@ -645,7 +662,7 @@ int ensure_rt_tc(cvad_engine *e, int src_rate, cudaStream_t stream) {
 // Does the model part of this step run as ONE fused kernel (the form cvad_step_device chains)?
 bool fused_single_frame(const cvad_engine *e, const cvad_step_args *a) {
     return e->chain_steps && e->version == CVAD_MODEL_V5 && e->math != CVAD_MATH_FP32 && a->max_frames == 1 && e->fuse_single_frame &&
-           a->channels <= 1;
+           a->channels <= 1 && !is_g711(a->pcm_format);
 }
 
 // a chained kernel sits at the tail of its stream without a `last_done` record: place the record now
@@ -659,8 +676,9 @@ int flush_chain(cvad_engine *e) {
 
 // AudioUtils.convert_to_mono (audio.py:193-208) on the device: out[i][k] = float32 mean over the C interleaved channels
 // of sample frame k of stream i -- the channels added in order, the sum divided by C, as np.mean does for float32 input.
-// PCM samples are converted to float first (the reference converts before it reaches the wrapper).  Per-stream rates:
-// stream i holds max_frames * 512 * src_rates[i] / 16000 sample frames.
+// PCM samples are converted to float first (the reference converts before it reaches the wrapper); G.711 codes are
+// decoded to linear / 32768, so with C == 1 this is the G.711 decode alone.  Per-stream rates: stream i holds
+// max_frames * 512 * src_rates[i] / 16000 sample frames.
 __global__ void downmix_kernel(const void *audio, int pcm, long long stride, int C, int n_streams, long long frames,
                                const int *src_rates, int max_frames, float *out) {
     for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < (long long)n_streams * frames;
@@ -673,7 +691,9 @@ __global__ void downmix_kernel(const void *audio, int pcm, long long stride, int
         for (int c = 0; c < C; ++c) {
             float x;
             if (pcm == 0) x = __ldg(reinterpret_cast<const float *>(audio) + base + c);
-            else {
+            else if (pcm >= CVAD_PCM_ULAW) {
+                x = (float)g711_linear(pcm, __ldg(reinterpret_cast<const unsigned char *>(audio) + base + c)) * (1.0f / 32768.0f);
+            } else {
                 x = (float)__ldg(reinterpret_cast<const short *>(audio) + base + c);
                 x = pcm == 1 ? __fdiv_rn(x, 32767.0f) : x * (1.0f / 32768.0f);
             }
@@ -690,20 +710,22 @@ int launch_step(cvad_engine *e, const cvad_step_args *a, unsigned int *d_status,
                 cudaStream_t stream, unsigned rates_mask = 0xFu, bool chain = false, const float **input_out = nullptr) {
     if (a->n_streams == 0 || a->max_frames == 0) return CVAD_OK;
     cvad_step_args a_mono;
-    if (a->channels > 1) {
-        // stage -1: interleaved channels -> mono float32 in HBM; everything downstream sees a mono float stream
-        if (chain) return fail(e, CVAD_E_INVALID, "internal: chained step with multi-channel input");
+    if (a->channels > 1 || is_g711(a->pcm_format)) {
+        // stage -1: interleaved channels and / or G.711 codes -> mono float32 in HBM; everything downstream sees a mono
+        // float stream
+        if (chain) return fail(e, CVAD_E_INVALID, "internal: chained step with multi-channel or G.711 input");
         int rcf = flush_chain(e);
         if (rcf) return rcf;
         CU_TRY(e, cudaStreamWaitEvent(stream, e->last_done, 0));     // d_mono is shared by consecutive steps
-        const long long frames = a->src_rates ? std::min<long long>((long long)a->max_frames * 1536, a->stream_stride / a->channels)
+        const int nch = std::max(a->channels, 1);
+        const long long frames = a->src_rates ? std::min<long long>((long long)a->max_frames * 1536, a->stream_stride / nch)
                                               : (long long)(a->max_frames - 1) * a->hop + a->frame_len;
         int rcg = grow(e, e->d_mono, (size_t)a->n_streams * (size_t)frames * sizeof(float));
         if (rcg) return rcg;
         if (input_out) CU_TRY(e, cudaMemsetAsync(e->d_mono.p, 0xFF, (size_t)a->n_streams * (size_t)frames * sizeof(float), stream));
         const long long total = (long long)a->n_streams * frames;
         const int grid = (int)std::min<long long>((total + 255) / 256, (long long)e->num_sms * 16);
-        downmix_kernel<<<grid, 256, 0, stream>>>(a->audio, a->pcm_format, a->stream_stride, a->channels, a->n_streams, frames,
+        downmix_kernel<<<grid, 256, 0, stream>>>(a->audio, a->pcm_format, a->stream_stride, nch, a->n_streams, frames,
                                                  a->src_rates, a->max_frames, static_cast<float *>(e->d_mono.p));
         CU_TRY(e, cudaGetLastError());
         e->launches++;
@@ -1074,11 +1096,13 @@ int quiesce(cvad_engine *e) {
 }
 
 // Floats cvad_debug_input writes for the (validated) step `a`: the d_res layout for resampled and mixed-rate steps,
-// the d_mono layout for down-mix-only steps; -1 = the step has no input stage (16 kHz mono).
+// the d_mono layout for 16 kHz steps with a down-mix or G.711 decode; -1 = the step has no input stage (16 kHz mono
+// float32 / int16).
 long long input_stage_floats(const cvad_step_args *a) {
     if (a->n_streams == 0 || a->max_frames == 0) return 0;
     if (a->src_rates || (a->src_rate != 0 && a->src_rate != 16000)) return (long long)a->n_streams * a->max_frames * 512;
-    if (a->channels > 1) return (long long)a->n_streams * ((long long)(a->max_frames - 1) * a->hop + a->frame_len);
+    if (a->channels > 1 || is_g711(a->pcm_format))
+        return (long long)a->n_streams * ((long long)(a->max_frames - 1) * a->hop + a->frame_len);
     return -1;
 }
 
@@ -1102,7 +1126,7 @@ int step_submit_impl(cvad_engine *e, cvad_engine::Lane &ln, const cvad_step_args
     if (rc) return rc;
     if (input_out) {
         const long long nf = input_stage_floats(a);
-        if (nf < 0) return fail(e, CVAD_E_INVALID, "cvad_debug_input: the step has no input stage (16 kHz mono)");
+        if (nf < 0) return fail(e, CVAD_E_INVALID, "cvad_debug_input: the step has no input stage (16 kHz mono float32 / int16)");
         if (input_floats < (size_t)nf) return fail(e, CVAD_E_CAPACITY, "cvad_debug_input: out too small");
     }
     CU_TRY(e, cudaSetDevice(e->device));

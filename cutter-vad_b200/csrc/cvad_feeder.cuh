@@ -97,6 +97,7 @@ struct cvad_feeder {
     int src_rate = 16000;              // 0 = per-slot rates (mixed)
     int max_step_frames = 8;           // frames one stream may run per step (a stream further behind catches up over steps)
     size_t es = 4;                     // bytes per sample
+    int64_t align = 8;                 // rows are whole multiples of this many samples: 16 bytes at least (feeder_copy_nt)
     size_t cap = 0;                    // arena row length (samples)
     unsigned char *arena = nullptr;    // pinned [max_streams][cap]
     std::mutex mu;                     // guards arena + fill + slot table (push vs step)
@@ -160,8 +161,24 @@ int ffail(cvad_feeder *f, int code, const std::string &msg) {
     return code;
 }
 
+// G.711 code -> decoded float32 sample (g711_linear / 32768), one 256-entry table per law
+struct G711Tables {
+    float t[2][256];
+    G711Tables() {
+        for (int c = 0; c < 256; ++c) {
+            t[0][c] = (float)g711_linear(CVAD_PCM_ULAW, (unsigned)c) / 32768.0f;
+            t[1][c] = (float)g711_linear(CVAD_PCM_ALAW, (unsigned)c) / 32768.0f;
+        }
+    }
+};
+inline const float *g711_table(int pcm) {
+    static const G711Tables tables;
+    return tables.t[pcm == CVAD_PCM_ALAW ? 1 : 0];
+}
+
 inline float feeder_sample(const cvad_feeder *f, const unsigned char *p, size_t k) {
     if (f->pcm_format == CVAD_PCM_F32) return reinterpret_cast<const float *>(p)[k];
+    if (is_g711(f->pcm_format)) return g711_table(f->pcm_format)[p[k]];
     const float v = (float)reinterpret_cast<const int16_t *>(p)[k];
     return f->pcm_format == CVAD_PCM_S16_32767 ? v / 32767.0f : v / 32768.0f;
 }
@@ -169,13 +186,16 @@ inline float feeder_sample(const cvad_feeder *f, const unsigned char *p, size_t 
 // numpy's `np.where(np.abs(f) > 0.01, f, 0.0)` on float32 data (audio.py:117-118): the threshold is float32(0.01)
 // One loop per sample format and gate setting, branch-free inside (the compiler vectorises them; the per-sample format
 // test of feeder_sample kept the 480-sample loop scalar: ~0.5 us per frame, most of the segment-assembly phase).
+// G.711 (FMT CVAD_PCM_ULAW, the same loop for both laws) reads its law's table `lut`.
 template <int FMT, bool GATE>
-inline void feeder_gate_loop(const unsigned char *__restrict__ src, int n, float *__restrict__ d) {
+inline void feeder_gate_loop(const unsigned char *__restrict__ src, int n, float *__restrict__ d,
+                             const float *__restrict__ lut = nullptr) {
     for (int k = 0; k < n; ++k) {
         float v;
         if (FMT == CVAD_PCM_F32) v = reinterpret_cast<const float *>(src)[k];
         else if (FMT == CVAD_PCM_S16_32767) v = (float)reinterpret_cast<const int16_t *>(src)[k] / 32767.0f;
-        else v = (float)reinterpret_cast<const int16_t *>(src)[k] / 32768.0f;
+        else if (FMT == CVAD_PCM_S16_32768) v = (float)reinterpret_cast<const int16_t *>(src)[k] / 32768.0f;
+        else v = lut[src[k]];
         d[k] = (!GATE || std::fabs(v) > 0.01f) ? v : 0.0f;
     }
 }
@@ -189,7 +209,12 @@ inline void feeder_gate_append(const cvad_feeder *f, const cvad_feeder::Slot &s,
         case CVAD_PCM_F32: g ? feeder_gate_loop<CVAD_PCM_F32, true>(src, n, d) : feeder_gate_loop<CVAD_PCM_F32, false>(src, n, d); break;
         case CVAD_PCM_S16_32767:
             g ? feeder_gate_loop<CVAD_PCM_S16_32767, true>(src, n, d) : feeder_gate_loop<CVAD_PCM_S16_32767, false>(src, n, d); break;
-        default: g ? feeder_gate_loop<CVAD_PCM_S16_32768, true>(src, n, d) : feeder_gate_loop<CVAD_PCM_S16_32768, false>(src, n, d); break;
+        case CVAD_PCM_S16_32768:
+            g ? feeder_gate_loop<CVAD_PCM_S16_32768, true>(src, n, d) : feeder_gate_loop<CVAD_PCM_S16_32768, false>(src, n, d); break;
+        default: {
+            const float *lut = g711_table(f->pcm_format);
+            g ? feeder_gate_loop<CVAD_PCM_ULAW, true>(src, n, d, lut) : feeder_gate_loop<CVAD_PCM_ULAW, false>(src, n, d, lut); break;
+        }
     }
 }
 
@@ -283,10 +308,10 @@ int feeder_gather(cvad_feeder *f, bool allow_planes = false) {
     f->tmax = tmax;
     if (n == 0) { f->row = 0; return CVAD_OK; }
     if (!mixed) row = (int64_t)(tmax - 1) * f->hop + f->frame_len;
-    row += (-row) & 7;                         // rows start 16-byte aligned in either sample format
+    row += (-row) & (f->align - 1);            // rows start 16-byte aligned in every sample format
     f->row = row;
     f->planes = allow_planes && !mixed && tmax >= 2 && tmax <= 4;
-    f->plane_row = ((int64_t)f->frame_len + 7) & ~(int64_t)7;
+    f->plane_row = ((int64_t)f->frame_len + f->align - 1) & ~(f->align - 1);
     size_t plane_rows = (size_t)n;
     if (f->planes) {
         f->ppos.assign((size_t)(tmax - 1) * (size_t)n, 0);
@@ -449,7 +474,7 @@ int cvad_feeder_create(cvad_engine *e, int max_streams, int pcm_format, int fram
     *out = nullptr;
     if (e) max_streams = e->max_streams;
     if (max_streams < 1) return fail(e, CVAD_E_INVALID, "feeder: max_streams < 1");
-    if (pcm_format < 0 || pcm_format > 2) return fail(e, CVAD_E_INVALID, "feeder: unknown pcm_format");
+    if (pcm_format < 0 || pcm_format > CVAD_PCM_ALAW) return fail(e, CVAD_E_INVALID, "feeder: unknown pcm_format");
     if (src_rate != 0 && src_rate != 16000) {
         if (rate_index(src_rate) < 0) return fail(e, CVAD_E_INVALID, "feeder: src_rate must be 0, 8000, 16000, 24000 or 48000");
         frame_len = hop = rate_n_in(src_rate);
@@ -464,11 +489,12 @@ int cvad_feeder_create(cvad_engine *e, int max_streams, int pcm_format, int fram
     f->frame_len = frame_len;
     f->hop = hop;
     f->src_rate = src_rate;
-    f->es = pcm_format == CVAD_PCM_F32 ? 4 : 2;
+    f->es = elem_size(pcm_format);
+    f->align = std::max<int64_t>(8, 16 / (int64_t)f->es);
     f->max_step_frames = capacity_frames;
     // rows start small (the arena is max_streams rows of pinned memory) and grow when a producer runs ahead of step()
     f->cap = (size_t)frame_len + (size_t)(std::min(capacity_frames, 3) + 1) * (size_t)std::max(hop, frame_len);
-    f->cap += (-(int64_t)f->cap) & 7;
+    f->cap += (-(int64_t)f->cap) & (f->align - 1);
     const size_t bytes = (size_t)max_streams * f->cap * f->es;
     if (e) {
         cudaSetDevice(e->device);
@@ -577,7 +603,7 @@ int64_t cvad_feeder_pending(cvad_feeder *f, int slot) {
 static int feeder_grow_arena(cvad_feeder *f, int64_t need) {
     if (need <= (int64_t)f->cap) return CVAD_OK;
     size_t cap = std::max<size_t>((size_t)need, 2 * f->cap);
-    cap += (-(int64_t)cap) & 7;
+    cap += (-(int64_t)cap) & (f->align - 1);
     const size_t bytes = (size_t)f->max_streams * cap * f->es;
     if (bytes > kFeederArenaLimit)
         return ffail(f, CVAD_E_CAPACITY, "stream buffer full: step() the feeder before pushing more audio");

@@ -9,7 +9,7 @@ that has at least one complete frame buffered, in ONE `cvad_step`:
 
     mgr = BatchedVADManager(max_streams=10_000)
     sid = mgr.open_stream(VADConfig(...), on_voice_start=..., on_voice_end=..., on_voice_continue=...)
-    mgr.push(sid, samples)            # float32 in [-1,1] or int16 PCM, any length
+    mgr.push(sid, samples)            # float32 in [-1,1], int16 PCM or G.711 bytes, any length
     out = mgr.step()                  # events in stream-then-frame order, callbacks fired
 
 Per stream the results equal what a `VADWrapper` fed the same frames would produce:
@@ -94,7 +94,8 @@ class BatchedVADManager:
         (`VADConfig.sample_rate` at open_stream, any of 8000 / 16000 / 24000 / 48000) and all of them
         advance in ONE engine step (cvad_step_args.src_rates), the way a websocket server meets them.
         `frames_per_step`: frames one stream runs per step at most; a stream that is further behind
-        catches up over the following steps."""
+        catches up over the following steps.  `pcm_format` capi.PCM_ULAW / PCM_ALAW: streams deliver G.711 bytes
+        (telephony), decoded on the GPU; callback payloads are the decoded float32 audio."""
         self.mixed = source_rate is None
         if self.mixed:
             source_rate, frame_len, hop = 48000, 1536, 1536        # arena sizing; per-stream values in the feeder
@@ -110,7 +111,8 @@ class BatchedVADManager:
         if self.hop < 1:
             raise ConfigurationError("hop", str(hop))
         self.pcm_format = pcm_format
-        self._dtype = np.float32 if pcm_format == capi.PCM_F32 else np.int16
+        self._dtype = capi.pcm_dtype(pcm_format).type
+        self._g711 = {capi.PCM_ULAW: "ulaw", capi.PCM_ALAW: "alaw"}.get(pcm_format)
         from ..engine.pool import default_device
         try:
             self._engine = StreamEngine(model_version.value, max_streams=max_streams,
@@ -219,9 +221,13 @@ class BatchedVADManager:
 
     # ------------------------------------------------------------------ data path
     def _check_samples(self, samples) -> np.ndarray:
+        if self._g711 and isinstance(samples, (bytes, bytearray, memoryview)):
+            samples = np.frombuffer(samples, np.uint8)
         x = np.asarray(samples)
         if x.size == 0:
             raise AudioProcessingError("Audio data is empty")
+        if self._g711 and x.dtype != np.uint8:
+            raise AudioProcessingError(f"G.711 audio must be uint8 codes or bytes, not {x.dtype}")
         return np.ascontiguousarray(x, dtype=self._dtype)
 
     @staticmethod
@@ -236,6 +242,9 @@ class BatchedVADManager:
         self._stream(stream_id)
         x = self._check_samples(samples)
         if x.ndim == 2:
+            if self._g711:
+                # the mean of G.711 codes is not the mean of the samples
+                raise AudioProcessingError("G.711 audio must be one channel: [samples] codes")
             x = np.ascontiguousarray(x.mean(axis=1).astype(self._dtype))
         try:
             self._feeder.push(stream_id, x)
@@ -268,7 +277,11 @@ class BatchedVADManager:
             self._raise(exc)
 
     def _gate(self, st: _Stream, frame: np.ndarray) -> np.ndarray:
-        f = frame.astype(np.float32)
+        if self._g711:
+            from ..utils.audio import AudioUtils
+            f = AudioUtils.g711_to_float32(frame, self._g711)
+        else:
+            f = frame.astype(np.float32)
         if self.pcm_format == capi.PCM_S16_32767:
             f = f / np.float32(32767.0)
         elif self.pcm_format == capi.PCM_S16_32768:

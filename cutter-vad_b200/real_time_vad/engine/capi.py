@@ -19,6 +19,7 @@ DEV_LIB_PATH = PKG_ROOT / "libcvad_b200_dev.so"     # development probes (csrc/c
 OK, E_INVALID, E_CUDA, E_NOGPU, E_WEIGHTS, E_CAPACITY = 0, -1, -2, -3, -4, -5
 MODEL_V5, MODEL_V4, MODEL_V4_8K = 5, 4, 48
 PCM_F32, PCM_S16_32767, PCM_S16_32768 = 0, 1, 2
+PCM_ULAW, PCM_ALAW = 3, 4                                   # G.711, one byte per sample, decoded on the GPU
 FLAG_STARTED, FLAG_ENDED, FLAG_CONTINUING = 1, 2, 4
 STATUS_NONFINITE = 1
 MATH_FP32, MATH_TC, MATH_TC16, MATH_FFT = 0, 1, 2, 3
@@ -87,6 +88,15 @@ class FeederResult(C.Structure):
                 ("n_events", C.c_int32), ("n_deliveries", C.c_int32), ("events", C.c_void_p),
                 ("deliveries", C.c_void_p), ("raw", C.c_void_p), ("raw_stride", C.c_int64),
                 ("gather_ms", C.c_double), ("gpu_ms", C.c_double), ("deliver_ms", C.c_double)]
+
+
+def pcm_dtype(pcm_format: int) -> np.dtype:
+    """numpy dtype of one sample in `pcm_format` (CVAD_PCM_*): float32, int16, or uint8 for the G.711 codes."""
+    if pcm_format == PCM_F32:
+        return np.dtype(np.float32)
+    if pcm_format in (PCM_ULAW, PCM_ALAW):
+        return np.dtype(np.uint8)
+    return np.dtype(np.int16)
 
 
 _lib = None

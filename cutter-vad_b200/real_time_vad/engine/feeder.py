@@ -69,7 +69,7 @@ def set_row_payloads(blob: bytes, payloads: Sequence[int]) -> bytes:
         magic, version, pcm, _fl, _hop, _sr, n, _z = struct.unpack_from("<IIiiiiii", b, 0)
         if magic != capi.FEEDER_SNAPSHOT_MAGIC or version != capi.FEEDER_SNAPSHOT_VERSION or n != len(payloads):
             raise ValueError("not a feeder snapshot with one row per stream")
-        es = 4 if pcm == capi.PCM_F32 else 2
+        es = capi.pcm_dtype(pcm).itemsize
         pos = 32
         for i in range(n):
             struct.pack_into("<i", b, pos + 8, int(payloads[i]))
@@ -104,7 +104,7 @@ class StreamFeeder:
             msg = (self._L.cvad_last_error(eh) or b"").decode() if eh is not None else "bad feeder arguments"
             raise FeederError(rc, msg)
         self.pcm_format = int(pcm_format)
-        self.dtype = np.float32 if pcm_format == capi.PCM_F32 else np.int16
+        self.dtype = capi.pcm_dtype(pcm_format).type
         self.max_streams = n
         self._res = capi.FeederResult()
 
@@ -168,7 +168,7 @@ class StreamFeeder:
 
     # ------------------------------------------------------------------ data path
     def push(self, slot: int, samples: np.ndarray) -> None:
-        """`samples`: 1-D contiguous array of the feeder's dtype."""
+        """`samples`: 1-D contiguous array of the feeder's dtype (uint8 codes for G.711)."""
         self._check(self._L.cvad_feeder_push(self._h, int(slot), samples.ctypes.data, samples.size))
 
     def push_bytes(self, slot: int, data: bytes) -> None:

@@ -250,10 +250,11 @@ class StreamEngine:
               src_rates=None):
         if audio.ndim not in (2, 3):
             raise EngineError(capi.E_INVALID, "audio must be [n_streams, samples] or [n_streams, samples, channels]")
-        if pcm_format == capi.PCM_F32:
-            audio = np.ascontiguousarray(audio, dtype=np.float32)
-        else:
-            audio = np.ascontiguousarray(audio, dtype=np.int16)
+        dtype = capi.pcm_dtype(pcm_format)
+        if dtype == np.uint8 and audio.dtype != np.uint8:
+            # G.711 codes are bytes: a cast from any other dtype would turn samples into meaningless codes
+            raise EngineError(capi.E_INVALID, f"G.711 audio must be uint8 codes, not {audio.dtype}")
+        audio = np.ascontiguousarray(audio, dtype=dtype)
         n = audio.shape[0]
         keep = [audio]
         a = capi.StepArgs()

@@ -25,6 +25,24 @@ from ..core.exceptions import AudioProcessingError
 _WINDOWS = {"hanning": np.hanning, "hamming": np.hamming, "blackman": np.blackman}
 
 
+def _g711_tables():
+    """ITU-T G.711 expansion of all 256 codes to 16-bit linear values (audioop.ulaw2lin / alaw2lin, width 2), the
+    same integer arithmetic as the engine's decode stage."""
+    c = np.arange(256, dtype=np.int32)
+    u = ~c & 0xFF
+    t = (((u & 0x0F) << 3) + 0x84) << ((u & 0x70) >> 4)
+    ulaw = np.where(u & 0x80, 0x84 - t, t - 0x84)
+    a = c ^ 0x55
+    seg = (a & 0x70) >> 4
+    t = (a & 0x0F) << 4
+    m = np.where(seg == 0, t + 8, (t + 0x108) << np.maximum(seg - 1, 0))
+    alaw = np.where(a & 0x80, m, -m)
+    return {"ulaw": ulaw.astype(np.int16), "alaw": alaw.astype(np.int16)}
+
+
+G711_LINEAR = _g711_tables()
+
+
 class AudioUtils:
     # ------------------------------------------------------------------ hot-path helpers
     @staticmethod
@@ -132,6 +150,17 @@ class AudioUtils:
             wavfile.write(file_path, sample_rate, AudioUtils._to_int(audio_data, bit_depth))
         except Exception as exc:
             raise AudioProcessingError(f"Failed to save audio file {file_path}: {exc}")
+
+    @staticmethod
+    def g711_to_float32(codes, law: str) -> np.ndarray:
+        """G.711 codes (uint8 array or bytes) -> float32 samples linear / 32768, with `law` "ulaw" or "alaw": exactly
+        pcm_to_float32 of the linear PCM, and exactly what the engine's decode stage produces."""
+        if law not in G711_LINEAR:
+            raise AudioProcessingError(f"unknown G.711 law {law!r}")
+        x = np.frombuffer(codes, np.uint8) if isinstance(codes, (bytes, bytearray, memoryview)) else np.asarray(codes)
+        if x.dtype != np.uint8:
+            raise AudioProcessingError(f"G.711 codes must be uint8, not {x.dtype}")
+        return G711_LINEAR[law][x].astype(np.float32) / np.float32(32768.0)
 
     @staticmethod
     def pcm_to_float32(pcm_data: bytes, bit_depth: int = 16) -> np.ndarray:

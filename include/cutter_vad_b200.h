@@ -78,10 +78,12 @@ extern "C" {
 #define CVAD_RESAMPLE_FFT 0   /* default: scipy.signal.resample's FFT method in double, rounded once to float32 */
 #define CVAD_RESAMPLE_GEMM 1  /* the dense operator R x (FP32 FMA or split-precision tensor cores, following cvad_set_math) */
 
-/* audio sample formats accepted by cvad_step */
+/* audio sample formats accepted by cvad_step, cvad_step_device and the stream feeder */
 #define CVAD_PCM_F32 0        /* float32 in [-1, 1] */
 #define CVAD_PCM_S16_32767 1  /* int16, divided by 32767.0f  (websocket server, vad_websocket_server.py:341) */
 #define CVAD_PCM_S16_32768 2  /* int16, divided by 32768.0f  (AudioUtils.pcm_to_float32, audio.py:308) */
+#define CVAD_PCM_ULAW 3       /* G.711 mu-law, one byte per sample: the ITU-T G.711 linear value (+-32124) / 32768.0f */
+#define CVAD_PCM_ALAW 4       /* G.711 A-law, one byte per sample: the ITU-T G.711 linear value (+-32256) / 32768.0f */
 
 /* per-frame flag bits written to flags_out (ProcessingResult, silero_model.py:99-113) */
 #define CVAD_FLAG_STARTED 1u
@@ -111,8 +113,10 @@ typedef struct cvad_step_args {
     int32_t n_streams;        /* number of slots stepped in this call (>= 0) */
     const int32_t *slots;     /* [n_streams] distinct slot ids; NULL = 0..n_streams-1 */
     const void *audio;        /* sample (i, k) at audio[i*stream_stride + k] (elements) */
-    int32_t pcm_format;       /* CVAD_PCM_* */
-    int64_t stream_stride;    /* elements between consecutive streams' first samples */
+    int32_t pcm_format;       /* CVAD_PCM_*.  CVAD_PCM_ULAW / CVAD_PCM_ALAW (one byte per sample) are decoded on the GPU by
+                                 the input stage before anything else; cvad_step_device runs such steps unchained
+                                 (memset + event record per step, like multi-channel steps) */
+    int64_t stream_stride;    /* elements between consecutive streams' first samples (bytes for G.711) */
     const int32_t *n_frames;  /* [n_streams] frames per stream (0..max_frames); NULL = max_frames each */
     int32_t max_frames;       /* row length of probs_out / flags_out */
     int32_t frame_len;        /* samples per frame before zero-padding/truncation to 512 (1..2048) */
@@ -284,14 +288,14 @@ int cvad_read_timing(cvad_engine *e, double *frontend_ms, double *recurrent_ms, 
 int cvad_debug_dump(cvad_engine *e, const cvad_step_args *a, float *dbg_out, size_t dbg_floats);
 
 /*
- * Test hook: run only the input stages of the step `a` describes (the down-mix of interleaved channels and the
- * resampler, or the pass-through of 16 kHz streams in a mixed-rate step), staged exactly as cvad_step stages it,
- * and copy to `out` (host) the float32 mono 16 kHz samples the model kernels would read:
- *   resampled or mixed-rate steps: [n_streams][max_frames * 512];
- *   down-mix only:                 [n_streams][(max_frames - 1) * hop + frame_len].
+ * Test hook: run only the input stages of the step `a` describes (the down-mix of interleaved channels or the G.711
+ * decode, and the resampler, or the pass-through of 16 kHz streams in a mixed-rate step), staged exactly as cvad_step
+ * stages it, and copy to `out` (host) the float32 mono 16 kHz samples the model kernels would read:
+ *   resampled or mixed-rate steps:     [n_streams][max_frames * 512];
+ *   down-mix or G.711 decode only:     [n_streams][(max_frames - 1) * hop + frame_len].
  * The device buffer is filled with 0xFF bytes (NaN) before the stages run, so a frame beyond a stream's n_frames
  * reads NaN in resampled output.  No model kernel runs and engine state is untouched.  Returns the number of floats
- * written, CVAD_E_CAPACITY if `n_floats` is too small, CVAD_E_INVALID for a step without an input stage (16 kHz mono).
+ * written, CVAD_E_CAPACITY if `n_floats` is too small, CVAD_E_INVALID for a step without an input stage (16 kHz mono float32 / int16).
  */
 int cvad_debug_input(cvad_engine *e, const cvad_step_args *a, float *out, size_t n_floats);
 
@@ -376,8 +380,9 @@ int cvad_feeder_clear(cvad_feeder *f, int slot);          /* VADProcessor.reset:
 int cvad_feeder_is_active(cvad_feeder *f, int slot);      /* host mirror of is_voice_active: 1 / 0 */
 int64_t cvad_feeder_pending(cvad_feeder *f, int slot);    /* samples buffered */
 
-/* Append samples (feeder's PCM format) to a slot.  float32 input containing NaN / Inf is rejected here, before any
-   state changes (AudioUtils.validate_audio_data, audio.py:227-228).  CVAD_E_CAPACITY when the arena cannot grow further. */
+/* Append samples (feeder's PCM format; bytes for G.711) to a slot.  float32 input containing NaN / Inf is rejected here,
+   before any state changes (AudioUtils.validate_audio_data, audio.py:227-228); every G.711 byte is a valid sample.
+   Voice-end segments and voice-continue frames of a G.711 feeder hold the decoded, gated float32 audio.  CVAD_E_CAPACITY when the arena cannot grow further. */
 int cvad_feeder_push(cvad_feeder *f, int slot, const void *samples, int64_t n_samples);
 /* block[i*row_stride .. +n_samples) is appended to slots[i]; all or nothing. */
 int cvad_feeder_push_many(cvad_feeder *f, int n, const int32_t *slots, const void *block, int64_t row_stride,
@@ -409,7 +414,8 @@ int cvad_feeder_deliver_only(cvad_feeder *f, const float *probs, const uint8_t *
  *       int32 rate, n_in (source samples per model frame), payload (CVAD_PAYLOAD_*), enable_denoising (0 / 1),
  *       float64 vad_start_probability, int32 voice active (the host mirror, 0 / 1), int32 0,
  *       int64 skip (hop > frame_len: samples still to drop from the next push), int64 n_pending, n_pre_roll, n_segment
- *   followed by n_pending samples in the feeder's PCM format, then n_pre_roll and n_segment float32 samples.
+ *   followed by n_pending samples in the feeder's PCM format (4, 2 or, for G.711, 1 byte each), then n_pre_roll and
+ *   n_segment float32 samples.
  */
 #define CVAD_FEEDER_SNAPSHOT_MAGIC 0x53465643u   /* "CVFS" */
 #define CVAD_FEEDER_SNAPSHOT_VERSION 1
