@@ -1714,6 +1714,11 @@ int cvad_get_state(cvad_engine *e, int slot, float *h, float *c, int32_t *sm, in
 int cvad_set_state(cvad_engine *e, int slot, const float *h, const float *c, const int32_t *sm) {
     if (!e) return CVAD_E_INVALID;
     if (slot < 0 || slot >= e->max_streams) return fail(e, CVAD_E_CAPACITY, "slot id out of range");
+    // the rule of cvad_import_states (validate_states_kernel), checked before anything is copied
+    if (h)
+        for (int j = 0; j < 128; ++j)
+            if (!(std::fabs(h[j]) <= 2.f))
+                return fail(e, CVAD_E_INVALID, "h[" + std::to_string(j) + "] is not within [-2, 2]; no state was changed");
     CU_TRY(e, cudaSetDevice(e->device));
     { int rcq = quiesce(e); if (rcq) return rcq; }
     const size_t pitch = 8 * sizeof(float), at = cvad::state_at(0, slot);

@@ -87,7 +87,9 @@ __global__ void validate_states_kernel(const cvad_stream_state *in, int n, unsig
     if (k >= n) return;
     const cvad_stream_state &r = in[k];
     bool ok = true;
-    for (int j = lane; j < 128; j += 32) ok = ok && isfinite(r.h[j]) && isfinite(r.c[j]);
+    // |h| <= 2: the FP16-split kernels store h * 2^14 (fused) or h scaled with max(|x|max, 1) (two-kernel form) in
+    // FP16, whose largest finite value is 65504; 2 * 2^14 = 2^15 is exact, and h = o * tanh(c) of any step is within 1
+    for (int j = lane; j < 128; j += 32) ok = ok && fabsf(r.h[j]) <= 2.f && isfinite(r.c[j]);
     if (lane == 0) {
         ok = ok && (r.is_voice_active == 0 || r.is_voice_active == 1) && r.voice_start_frame_count >= 0 &&
              r.voice_end_frame_count >= 0 && r.frames_done >= 0 && r.vad_start_probability >= 0.0 &&
@@ -209,7 +211,7 @@ int cvad_import_states(cvad_engine *e, int n, const int32_t *slots, const cvad_s
     CU_TRY(e, cudaStreamSynchronize(e->stream));
     if (bad != kNoBadRecord)
         return fail(e, CVAD_E_INVALID, "import: record " + std::to_string(bad) +
-                    " is invalid (h and c must be finite, is_voice_active and enable_denoising 0 or 1, counts and"
+                    " is invalid (h within [-2, 2], c finite, is_voice_active and enable_denoising 0 or 1, counts and"
                     " frames_done >= 0, probabilities within [0, 1], n_start and n_end >= 1); no slot was changed");
     // 3. all passed: scatter
     import_states_kernel<<<state_grid(e, n), 256, 0, e->stream>>>(state_arrays(e), ds, n,

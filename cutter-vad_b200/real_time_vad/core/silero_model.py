@@ -28,8 +28,8 @@ from ..engine import ort_compat as ort
 from ..utils.audio import AudioUtils
 from ..utils.wav_writer import WAVWriter
 from .config import SampleRate, SileroModelVersion, VADConfig  # noqa: F401
-from .exceptions import (AudioProcessingError, CallbackError, ModelInitializationError,  # noqa: F401
-                         ModelNotFoundError, VADError)
+from .exceptions import (AudioProcessingError, CallbackError, ConfigurationError,  # noqa: F401
+                         ModelInitializationError, ModelNotFoundError, VADError)
 
 FRAME = 512                    # samples the model consumes per call (silero_model.py:464-471)
 START_WINDOW_CAP = 20          # deque(maxlen=20)  (silero_model.py:620-623)
@@ -495,6 +495,10 @@ class VADProcessor(BaseModel):
                 h_in, c_in = ms.state[0, 0].copy(), ms.state[1, 0].copy()
             else:
                 h_in, c_in = ms.hidden_state.reshape(128).copy(), ms.cell_state.reshape(128).copy()
+            if not (np.abs(h_in) <= ort.H_BOUND).all():
+                # a hand-set model_state the engine refuses (cvad_set_state): no LSTM step produces one
+                raise ConfigurationError("model_state", "h outside [-2, 2]",
+                                         "LSTM state h must lie within [-2, 2] (an LSTM's h stays within [-1, 1])")
             r, h, c, sm_out = run(first, count, h_in, c_in, sm_in)
             probs = r.probs[0]
             flags = r.flags[0]

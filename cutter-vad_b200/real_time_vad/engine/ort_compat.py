@@ -55,6 +55,9 @@ def get_device() -> str:
     return "GPU"
 
 
+# the largest |h| cvad_set_state / cvad_import_states accept (include/cutter_vad_b200.h)
+H_BOUND = 2.0
+
 _V5_MARK = "If_0_then_branch__Inline_0__stft.forward_basis_buffer"
 _V4_MARK = "model.feature_extractor.forward_basis_buffer"
 
@@ -150,6 +153,9 @@ class InferenceSession:
             if h_in.shape != (2, 1, 64) or c_in.shape != (2, 1, 64):
                 raise ValueError(f"h and c must have shape (2, 1, 64), got {h_in.shape} / {c_in.shape}")
             h_in, c_in = h_in.reshape(128), c_in.reshape(128)      # engine rows: layer-major [2][64]
+        if not (np.abs(h_in) <= H_BOUND).all():
+            raise ValueError(f"h must lie within [-{H_BOUND:g}, {H_BOUND:g}] (an LSTM's h = o * tanh(c) stays within "
+                             "[-1, 1]; the engine's FP16-split kernels cannot hold more)")
         eng = pooled.engine
         with pooled.lock:
             if pooled is self._pooled:

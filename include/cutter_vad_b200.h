@@ -193,7 +193,9 @@ int cvad_configure(cvad_engine *e, int n, const int32_t *slots, double vad_start
                    int voice_end_frame_count, int enable_denoising);
 
 /* LSTM state of one slot: h[128], c[128] for v5; h[2*64], c[2*64] for v4.
-   sm[4] = {is_voice_active, voice_start_frame_count, voice_end_frame_count, reserved}. */
+   sm[4] = {is_voice_active, voice_start_frame_count, voice_end_frame_count, reserved}.
+   cvad_set_state refuses an h outside [-2, 2] (NaN included) with CVAD_E_INVALID before it writes anything: the FP16-split
+   tensor-core kernels hold |h| <= 2 exactly, and an LSTM's own h = o * tanh(c) never leaves [-1, 1]. */
 int cvad_get_state(cvad_engine *e, int slot, float *h, float *c, int32_t *sm, int64_t *frames_done);
 int cvad_set_state(cvad_engine *e, int slot, const float *h, const float *c, const int32_t *sm);
 
@@ -221,8 +223,8 @@ int cvad_model_fingerprint(const cvad_engine *e, uint64_t *out);
    on another stream must be complete before cvad_import_states, and exported records are complete when it returns.
    Both wait for the steps
    in flight first and synchronise before returning, like cvad_reset, so the next step (chained device steps included)
-   reads the imported state.  Import is all or nothing: every record is checked on the device first (h and c finite,
-   is_voice_active and enable_denoising 0 or 1, counts and frames_done >= 0, probabilities in [0, 1], n_start and
+   reads the imported state.  Import is all or nothing: every record is checked on the device first (h within [-2, 2],
+   which the FP16-split tensor-core kernels hold exactly and which no LSTM step leaves; c finite; is_voice_active and enable_denoising 0 or 1, counts and frames_done >= 0, probabilities in [0, 1], n_start and
    n_end >= 1); one bad record fails the call with CVAD_E_INVALID, cvad_last_error names its index, and no slot changes.
    CVAD_E_CAPACITY: a slot id out of range; CVAD_E_INVALID: a slot listed twice. */
 int cvad_export_states(cvad_engine *e, int n, const int32_t *slots, cvad_stream_state *out);

@@ -206,6 +206,7 @@ def test_a_tc16_stream_continues_in_fp32_math_within_the_parity_bar():
 def _bad_records():
     yield "h NaN", lambda r: r["h"].__setitem__(5, np.nan)
     yield "c Inf", lambda r: r["c"].__setitem__(127, np.inf)
+    yield "|h| > 2", lambda r: r["h"].__setitem__(64, np.nextafter(np.float32(-2), np.float32(-3)))
     yield "active 2", lambda r: r.__setitem__("is_voice_active", 2)
     yield "start count < 0", lambda r: r.__setitem__("voice_start_frame_count", -1)
     yield "end count < 0", lambda r: r.__setitem__("voice_end_frame_count", -3)

@@ -207,16 +207,28 @@ def test_nonfinite_stream_is_rejected_without_state_change(engine_factory, ref_v
     assert np.abs(got - want).max() <= TOL
 
 
-def test_set_state_reset_and_errors(engine_factory):
+def test_set_state_within_the_h_bound_reset_and_errors(engine_factory):
+    """cvad_set_state writes any h within [-2, 2] (both ends included) and any c exactly; an h beyond the bound, or a
+    NaN, is refused before anything is written (the FP16-split kernels cannot hold it)."""
+    from real_time_vad.engine import capi
     from real_time_vad.engine.stream_engine import EngineError
     eng = engine_factory(128)
     eng.reset()
     rng = np.random.default_rng(1)
-    h = rng.standard_normal(128).astype(np.float32)
+    h = np.clip(rng.standard_normal(128), -2, 2).astype(np.float32)
+    h[:2] = 2.0, -2.0
     c = rng.standard_normal(128).astype(np.float32)
     eng.set_state(100, h, c, np.array([1, 2, 3, 0], np.int32))
     h2, c2, sm, _ = eng.get_state(100)
     assert np.array_equal(h, h2) and np.array_equal(c, c2) and sm[:3].tolist() == [1, 2, 3]
+    for bad in (np.nextafter(np.float32(2), np.float32(3)), -4.0, np.nan):
+        hb = h.copy()
+        hb[77] = bad
+        with pytest.raises(EngineError) as ei:
+            eng.set_state(100, hb, np.zeros(128, np.float32), np.zeros(4, np.int32))
+        assert ei.value.code == capi.E_INVALID and "h[77]" in ei.value.message
+        h2, c2, sm, _ = eng.get_state(100)
+        assert np.array_equal(h, h2) and np.array_equal(c, c2) and sm[:3].tolist() == [1, 2, 3]
     eng.reset([100])
     h2, c2, sm, _ = eng.get_state(100)
     assert not h2.any() and not c2.any() and not sm.any()
