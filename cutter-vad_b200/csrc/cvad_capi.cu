@@ -1,7 +1,7 @@
 // cvad_capi.cu -- host side of the C ABI declared in include/cutter_vad_b200.h.
 //
-// Owns: the engine object (one GPU, one stream), weight repacking into the kernels'
-// streaming layout, the per-slot state arena in HBM, per-step scratch buffers and the
+// Owns: the engine object (one GPU, one stream), the upload of the weight streams that
+// cvad_pack.cuh packs, the per-slot state arena in HBM, per-step scratch buffers and the
 // pinned staging used by the host-buffer entry point.  There is no CPU fallback: if no
 // sm_100 device is present every compute entry point fails with CVAD_E_NOGPU.
 #include <algorithm>
@@ -22,6 +22,7 @@
 #include "cvad_v4tc.cuh"
 #include "cvad_fftk.cuh"
 #include "cvad_v5tc.cuh"
+#include "cvad_pack.cuh"
 
 namespace {
 
@@ -152,385 +153,6 @@ bool is_host_pinned_or_device(const void *p, bool want_device) {
     return at.type == cudaMemoryTypeHost;
 }
 
-// ---- v5 weight repack (canonical blob order: see include/ and oracle/silero_ref.c)
-struct V5Packed {
-    std::vector<float> w_fe, b_fe, w_rec, b_rec, w_dec;
-};
-
-V5Packed pack_v5(const float *blob) {
-    const float *basis = blob;                       // [258][256]
-    const float *e0w = basis + 258 * 256;            // [128][129][3]
-    const float *e0b = e0w + 128 * 129 * 3;
-    const float *e1w = e0b + 128;                    // [64][128][3]
-    const float *e1b = e1w + 64 * 128 * 3;
-    const float *e2w = e1b + 64;                     // [64][64][3]
-    const float *e2b = e2w + 64 * 64 * 3;
-    const float *e3w = e2b + 64;                     // [128][64][3]
-    const float *e3b = e3w + 128 * 64 * 3;
-    const float *wih = e3b + 128;                    // [512][128]
-    const float *whh = wih + 512 * 128;
-    const float *bih = whh + 512 * 128;
-    const float *bhh = bih + 512;
-    const float *decw = bhh + 512;                   // [128]
-    const float *decb = decw + 128;
-
-    V5Packed P;
-    P.w_fe.assign(cvad::kFeStreamFloats, 0.f);
-    float *o = P.w_fe.data();
-    for (int k = 0; k < 256; ++k)
-        for (int n = 0; n < 256; ++n) {
-            int row;
-            if (n == 0) row = 0;
-            else if (n == 1) row = 128;
-            else row = (n & 1) ? 129 + (n >> 1) : (n >> 1);
-            o[k * 256 + n] = basis[row * 256 + k];
-        }
-    o += 65536;
-    for (int c = 0; c < 129; ++c)
-        for (int t = 0; t < 3; ++t)
-            for (int oc = 0; oc < 128; ++oc) o[(c * 3 + t) * 128 + oc] = e0w[(oc * 129 + c) * 3 + t];
-    o += 129 * 384;
-    for (int c = 0; c < 128; ++c)
-        for (int t = 0; t < 3; ++t)
-            for (int oc = 0; oc < 64; ++oc) o[(c * 3 + t) * 64 + oc] = e1w[(oc * 128 + c) * 3 + t];
-    o += 128 * 192;
-    for (int c = 0; c < 64; ++c)
-        for (int t = 0; t < 2; ++t)
-            for (int oc = 0; oc < 64; ++oc) o[(c * 2 + t) * 64 + oc] = e2w[(oc * 64 + c) * 3 + (t + 1)];
-    o += 64 * 128;
-    for (int c = 0; c < 64; ++c)
-        for (int oc = 0; oc < 128; ++oc) o[c * 128 + oc] = e3w[(oc * 64 + c) * 3 + 1];
-
-    P.b_fe.resize(cvad::kFeBiasFloats);
-    std::memcpy(P.b_fe.data(), e0b, 128 * 4);
-    std::memcpy(P.b_fe.data() + 128, e1b, 64 * 4);
-    std::memcpy(P.b_fe.data() + 192, e2b, 64 * 4);
-    std::memcpy(P.b_fe.data() + 256, e3b, 128 * 4);
-
-    P.w_rec.resize(cvad::kRecStreamFloats);
-    P.b_rec.resize(512);
-    for (int n = 0; n < 512; ++n) {
-        const int unit = n >> 2, gate = n & 3;
-        const int row = gate * 128 + unit;
-        for (int k = 0; k < 128; ++k) {
-            P.w_rec[k * 512 + n] = wih[row * 128 + k];
-            P.w_rec[(128 + k) * 512 + n] = whh[row * 128 + k];
-        }
-        P.b_rec[n] = bih[row] + bhh[row];
-    }
-    P.w_dec.resize(129);
-    std::memcpy(P.w_dec.data(), decw, 128 * 4);
-    P.w_dec[128] = decb[0];
-    return P;
-}
-
-
-// ---- v5 tensor-core repack: every GEMM weight as three BF16 parts (w = w0 + w1 + w2 to 24 bits), cut into
-// (rows x 64 K) tiles in the SWIZZLE_128B K-major operand layout, in the order cvad_v5tc.cuh consumes them.
-struct V5TcPacked {
-    std::vector<unsigned char> w_fe, w_rec;
-    std::vector<float> nyq_w, b_rec;
-};
-
-uint16_t bf16_rn_bits(float x) {
-    uint32_t u;
-    std::memcpy(&u, &x, 4);
-    const uint32_t r = ((u >> 16) & 1u) + 0x7FFFu;
-    return (uint16_t)((u + r) >> 16);
-}
-float bf16_val(uint16_t b) {
-    const uint32_t u = (uint32_t)b << 16;
-    float f;
-    std::memcpy(&f, &u, 4);
-    return f;
-}
-
-// append the three part tiles of W(row, k), rows x [k0, k0 + 64)
-template <typename F>
-void emit_tiles(std::vector<unsigned char> &out, int rows, int k0, F W) {
-    const size_t tile = (size_t)rows * 128;
-    const size_t at = out.size();
-    out.resize(at + 3 * tile, 0);
-    for (int r = 0; r < rows; ++r)
-        for (int kk = 0; kk < 64; ++kk) {
-            float x = W(r, k0 + kk);
-            const size_t off = (size_t)(r >> 3) * 1024 + (size_t)(r & 7) * 128 + (size_t)((((kk >> 3) ^ r) & 7) << 4) + (size_t)(kk & 7) * 2;
-            for (int part = 0; part < 3; ++part) {
-                const uint16_t b = bf16_rn_bits(x);
-                std::memcpy(&out[at + part * tile + off], &b, 2);
-                x -= bf16_val(b);
-            }
-        }
-}
-
-V5TcPacked pack_v5_tc(const float *blob) {
-    const float *basis = blob;                       // [258][256]
-    const float *e0w = basis + 258 * 256;            // [128][129][3]
-    const float *e0b = e0w + 128 * 129 * 3;
-    const float *e1w = e0b + 128;                    // [64][128][3]
-    const float *e1b = e1w + 64 * 128 * 3;
-    const float *e2w = e1b + 64;                     // [64][64][3]
-    const float *e2b = e2w + 64 * 64 * 3;
-    const float *e3w = e2b + 64;                     // [128][64][3]
-    const float *e3b = e3w + 128 * 64 * 3;
-    const float *wih = e3b + 128;                    // [512][128]
-    const float *whh = wih + 512 * 128;
-    const float *bih = whh + 512 * 128;
-    const float *bhh = bih + 512;
-
-    V5TcPacked P;
-    P.w_fe.reserve(cvad::tc5::kFeStreamBytes);
-    for (int blk = 0; blk < 2; ++blk)
-        for (int kb = 0; kb < 4; ++kb)
-            emit_tiles(P.w_fe, 128, kb * 64, [&](int m, int k) {
-                const int row = blk == 0 ? m : (m == 0 ? 128 : 129 + m);
-                return basis[row * 256 + k];
-            });
-    static const int taps0[3] = {1, 0, 2}, taps1[3] = {1, 2, 0};
-    for (int kb = 0; kb < 2; ++kb)
-        for (int ti = 0; ti < 3; ++ti)
-            emit_tiles(P.w_fe, 128, kb * 64, [&](int o, int c) { return e0w[(o * 129 + c) * 3 + taps0[ti]]; });
-    for (int kb = 0; kb < 2; ++kb)
-        for (int ti = 0; ti < 3; ++ti)
-            emit_tiles(P.w_fe, 64, kb * 64, [&](int o, int c) { return e1w[(o * 128 + c) * 3 + taps1[ti]]; });
-    for (int tap = 1; tap <= 2; ++tap)
-        emit_tiles(P.w_fe, 64, 0, [&](int o, int c) { return e2w[(o * 64 + c) * 3 + tap]; });
-    emit_tiles(P.w_fe, 128, 0, [&](int o, int c) { return e3w[(o * 64 + c) * 3 + 1]; });
-
-    for (int g = 0; g < 4; ++g)
-        for (int kb = 0; kb < 4; ++kb)
-            emit_tiles(P.w_rec, 128, kb * 64, [&](int u, int k) {
-                const int row = g * 128 + u;
-                return k < 128 ? wih[row * 128 + k] : whh[row * 128 + (k - 128)];
-            });
-
-    P.nyq_w.assign(128 * 4, 0.f);
-    for (int o = 0; o < 128; ++o)
-        for (int t = 0; t < 3; ++t) P.nyq_w[o * 4 + t] = e0w[(o * 129 + 128) * 3 + t];
-    P.b_rec.resize(512);
-    for (int n = 0; n < 512; ++n) P.b_rec[n] = bih[n] + bhh[n];
-    return P;
-}
-
-// ---- v5 FP16-split repack (CVAD_MATH_TC16): the same tile order with TWO FP16 parts per weight, every layer scaled
-// by the power of two that brings its largest weight to [2^14, 2^15) (inverse returned in inv_w: stft, enc0..3, W_ih, W_hh)
-struct V5HPacked {
-    std::vector<unsigned char> w_fe, w_rec;
-    float inv_w[8] = {0};
-};
-
-template <typename F>
-void emit_tiles_h(std::vector<unsigned char> &out, int rows, int k0, float scale, F W) {
-    const size_t tile = (size_t)rows * 128;
-    const size_t at = out.size();
-    out.resize(at + 2 * tile, 0);
-    for (int r = 0; r < rows; ++r)
-        for (int kk = 0; kk < 64; ++kk) {
-            float x = W(r, k0 + kk) * scale;
-            const size_t off = (size_t)(r >> 3) * 1024 + (size_t)(r & 7) * 128 + (size_t)((((kk >> 3) ^ r) & 7) << 4) + (size_t)(kk & 7) * 2;
-            for (int part = 0; part < 2; ++part) {
-                const __half h = __float2half_rn(x);
-                const unsigned short b = __half_as_ushort(h);
-                std::memcpy(&out[at + part * tile + off], &b, 2);
-                x -= __half2float(h);
-            }
-        }
-}
-
-float pow2_scale_for(float maxabs, float *inv) {
-    if (!(maxabs > 0.f)) { *inv = 1.f; return 1.f; }
-    int ex;
-    std::frexp(maxabs, &ex);                 // maxabs = m * 2^ex, m in [0.5, 1)  ->  maxabs in [2^(ex-1), 2^ex)
-    const float s = std::ldexp(1.0f, 15 - ex);
-    *inv = std::ldexp(1.0f, ex - 15);
-    return s;
-}
-
-V5HPacked pack_v5_tc16(const float *blob) {
-    const float *basis = blob;                       // [258][256]
-    const float *e0w = basis + 258 * 256;            // [128][129][3]
-    const float *e0b = e0w + 128 * 129 * 3;
-    const float *e1w = e0b + 128;                    // [64][128][3]
-    const float *e1b = e1w + 64 * 128 * 3;
-    const float *e2w = e1b + 64;                     // [64][64][3]
-    const float *e2b = e2w + 64 * 64 * 3;
-    const float *e3w = e2b + 64;                     // [128][64][3]
-    const float *e3b = e3w + 128 * 64 * 3;
-    const float *wih = e3b + 128;                    // [512][128]
-    const float *whh = wih + 512 * 128;
-    auto maxabs = [](const float *w, size_t n) { float m = 0.f; for (size_t i = 0; i < n; ++i) m = std::max(m, std::fabs(w[i])); return m; };
-    V5HPacked P;
-    const float s_stft = pow2_scale_for(maxabs(basis, 258 * 256), &P.inv_w[0]);
-    const float s_e0 = pow2_scale_for(maxabs(e0w, 128 * 129 * 3), &P.inv_w[1]);
-    const float s_e1 = pow2_scale_for(maxabs(e1w, 64 * 128 * 3), &P.inv_w[2]);
-    const float s_e2 = pow2_scale_for(maxabs(e2w, 64 * 64 * 3), &P.inv_w[3]);
-    const float s_e3 = pow2_scale_for(maxabs(e3w, 128 * 64 * 3), &P.inv_w[4]);
-    // one scale for [W_ih | W_hh]: the recurrent kernel accumulates both halves of K in the same TMEM columns
-    const float s_ih = pow2_scale_for(std::max(maxabs(wih, 512 * 128), maxabs(whh, 512 * 128)), &P.inv_w[5]);
-    const float s_hh = s_ih;
-    P.inv_w[6] = P.inv_w[5];
-    P.w_fe.reserve(cvad::tc5::kFeStreamBytesH);
-    for (int blk = 0; blk < 2; ++blk)
-        for (int kb = 0; kb < 4; ++kb)
-            emit_tiles_h(P.w_fe, 128, kb * 64, s_stft, [&](int m, int k) {
-                const int row = blk == 0 ? m : (m == 0 ? 128 : 129 + m);
-                return basis[row * 256 + k];
-            });
-    static const int taps0[3] = {1, 0, 2}, taps1[3] = {1, 2, 0};
-    for (int kb = 0; kb < 2; ++kb)
-        for (int ti = 0; ti < 3; ++ti)
-            emit_tiles_h(P.w_fe, 128, kb * 64, s_e0, [&](int o, int c) { return e0w[(o * 129 + c) * 3 + taps0[ti]]; });
-    for (int kb = 0; kb < 2; ++kb)
-        for (int ti = 0; ti < 3; ++ti)
-            emit_tiles_h(P.w_fe, 64, kb * 64, s_e1, [&](int o, int c) { return e1w[(o * 128 + c) * 3 + taps1[ti]]; });
-    for (int tap = 1; tap <= 2; ++tap)
-        emit_tiles_h(P.w_fe, 64, 0, s_e2, [&](int o, int c) { return e2w[(o * 64 + c) * 3 + tap]; });
-    emit_tiles_h(P.w_fe, 128, 0, s_e3, [&](int o, int c) { return e3w[(o * 64 + c) * 3 + 1]; });
-    for (int g = 0; g < 4; ++g)
-        for (int kb = 0; kb < 4; ++kb)
-            emit_tiles_h(P.w_rec, 128, kb * 64, kb < 2 ? s_ih : s_hh, [&](int u, int k) {
-                const int row = g * 128 + u;
-                return k < 128 ? wih[row * 128 + k] : whh[row * 128 + (k - 128)];
-            });
-    return P;
-}
-
-// v4 tensor-core STFT: the basis as 24 BF16x3 tiles (same row packing as v5's STFT block of pack_v5_tc)
-std::vector<unsigned char> pack_v4_stft_tc(const float *blob) {
-    const float *basis = blob;   // [258][256]
-    std::vector<unsigned char> out;
-    out.reserve(cvad::tc5::kV4StftStreamBytes);
-    for (int blk = 0; blk < 2; ++blk)
-        for (int kb = 0; kb < 4; ++kb)
-            emit_tiles(out, 128, kb * 64, [&](int m, int k) {
-                const int row = blk == 0 ? m : (m == 0 ? 128 : 129 + m);
-                return basis[row * 256 + k];
-            });
-    return out;
-}
-
-// v4 FFT path: delta = (the file's float32 STFT basis) - (periodic Hann x DFT-256, evaluated in double) -- what the
-// exact-basis FFT lacks.  Scaled by 2^24 it is O(1) and goes to the tensor cores as ONE BF16 part per weight
-// (8 tiles, blk x kb, same row packing as pack_v4_stft_tc).  Returns max |delta| (7.7e-8 for the reference's file).
-double pack_v4_stft_corr(const float *blob, const double2 *T, std::vector<unsigned char> &out) {
-    const float *basis = blob;   // [258][256]: rows 0..128 real part, 129..257 imaginary part (-sin)
-    double worst = 0.0;
-    std::vector<float> delta(258 * 256);
-    for (int row = 0; row < 258; ++row) {
-        const int k = row < 129 ? row : row - 129;
-        for (int n = 0; n < 256; ++n) {
-            const double2 w = T[6 * ((k * n) & 255)];                 // exp(-2 pi i k n / 256)
-            const double hann = 0.5 - 0.5 * T[6 * n].x;
-            const double exact = hann * (row < 129 ? w.x : w.y);
-            const double d = (double)basis[row * 256 + n] - exact;
-            worst = std::max(worst, std::fabs(d));
-            delta[row * 256 + n] = (float)(d * 16777216.0);
-        }
-    }
-    out.clear();
-    out.reserve(cvad::tc5::kV4CorrStreamBytes);
-    for (int blk = 0; blk < 2; ++blk)
-        for (int kb = 0; kb < 4; ++kb) {
-            const size_t tile = 128 * 128, at = out.size();
-            out.resize(at + tile, 0);
-            for (int r = 0; r < 128; ++r)
-                for (int kk = 0; kk < 64; ++kk) {
-                    const int row = blk == 0 ? r : (r == 0 ? 128 : 129 + r);
-                    const uint16_t b = bf16_rn_bits(delta[row * 256 + kb * 64 + kk]);
-                    const size_t off = (size_t)(r >> 3) * 1024 + (size_t)(r & 7) * 128 + (size_t)((((kk >> 3) ^ r) & 7) << 4) + (size_t)(kk & 7) * 2;
-                    std::memcpy(&out[at + off], &b, 2);
-                }
-        }
-    return worst;
-}
-
-// ---- v4 weight repack (canonical blob order: oracle/silero_ref.c "Silero VAD v4")
-V5Packed pack_v4(const float *blob) {
-    const float *p = blob;
-    auto take = [&](size_t n) { const float *r = p; p += n; return r; };
-    const float *basis = take(258 * 256), *nfilt = take(7);
-    const float *f_dw = take(258 * 5), *f_dwb = take(258), *f_pw = take(16 * 258), *f_pwb = take(16),
-                *f_pj = take(16 * 258), *f_pjb = take(16);
-    const float *c1 = take(256), *c1b = take(16);
-    const float *e3_dw = take(80), *e3_dwb = take(16), *e3_pw = take(512), *e3_pwb = take(32), *e3_pj = take(512),
-                *e3_pjb = take(32);
-    const float *c2 = take(1024), *c2b = take(32);
-    const float *e7_dw = take(160), *e7_dwb = take(32), *e7_pw = take(1024), *e7_pwb = take(32);
-    const float *c3 = take(1024), *c3b = take(32);
-    const float *e11_dw = take(160), *e11_dwb = take(32), *e11_pw = take(2048), *e11_pwb = take(64),
-                *e11_pj = take(2048), *e11_pjb = take(64);
-    const float *c4 = take(4096), *c4b = take(64);
-    const float *l1w = take(16384), *l1r = take(16384), *l1b = take(512);
-    const float *l2w = take(16384), *l2r = take(16384), *l2b = take(512);
-    const float *decw = take(64), *decb = take(1);
-
-    V5Packed P;
-    P.w_fe.assign(cvad::kV4FeStreamFloats, 0.f);
-    float *o = P.w_fe.data();
-    for (int k = 0; k < 256; ++k)
-        for (int n = 0; n < 256; ++n) {
-            int row;
-            if (n == 0) row = 0;
-            else if (n == 1) row = 128;
-            else row = (n & 1) ? 129 + (n >> 1) : (n >> 1);
-            o[k * 256 + n] = basis[row * 256 + k];
-        }
-    o = P.w_fe.data() + cvad::kV4OffFirst;
-    for (int c = 0; c < 258; ++c) {
-        float *r = o + c * 40;
-        for (int d = 0; d < 5; ++d) r[d] = f_dw[c * 5 + d];
-        r[5] = f_dwb[c];
-        for (int oc = 0; oc < 16; ++oc) { r[8 + oc] = f_pw[oc * 258 + c]; r[24 + oc] = f_pj[oc * 258 + c]; }
-    }
-    auto put_T = [](float *dst, const float *w, int cout, int cin) {  // w[co][ci] -> dst[ci][co]
-        for (int co = 0; co < cout; ++co)
-            for (int ci = 0; ci < cin; ++ci) dst[ci * cout + co] = w[co * cin + ci];
-    };
-    auto put_dw = [](float *dst, const float *w, int c) {             // w[c][5] -> dst[5][c]
-        for (int ch = 0; ch < c; ++ch)
-            for (int d = 0; d < 5; ++d) dst[d * c + ch] = w[ch * 5 + d];
-    };
-    o = P.w_fe.data() + cvad::kV4OffS0;
-    put_T(o, c1, 16, 16); std::memcpy(o + 256, c1b, 64);
-    put_dw(o + 272, e3_dw, 16); std::memcpy(o + 352, e3_dwb, 64);
-    put_T(o + 368, e3_pw, 32, 16); std::memcpy(o + 880, e3_pwb, 128);
-    put_T(o + 912, e3_pj, 32, 16); std::memcpy(o + 1424, e3_pjb, 128);
-    put_T(o + 1456, c2, 32, 32); std::memcpy(o + 2480, c2b, 128);
-    o = P.w_fe.data() + cvad::kV4OffS1;
-    put_dw(o, e7_dw, 32); std::memcpy(o + 160, e7_dwb, 128);
-    put_T(o + 192, e7_pw, 32, 32); std::memcpy(o + 1216, e7_pwb, 128);
-    put_T(o + 1248, c3, 32, 32); std::memcpy(o + 2272, c3b, 128);
-    o = P.w_fe.data() + cvad::kV4OffS2;
-    put_dw(o, e11_dw, 32); std::memcpy(o + 160, e11_dwb, 128);
-    put_T(o + 192, e11_pw, 64, 32); std::memcpy(o + 2240, e11_pwb, 256);
-    o = P.w_fe.data() + cvad::kV4OffS3;
-    put_T(o, e11_pj, 64, 32); std::memcpy(o + 2048, e11_pjb, 256); std::memcpy(o + 2112, c4b, 256);
-    o = P.w_fe.data() + cvad::kV4OffS4;
-    put_T(o, c4, 64, 64);
-    o = P.w_fe.data() + cvad::kV4OffMisc;
-    for (int oc = 0; oc < 16; ++oc) o[oc] = f_pwb[oc] + f_pjb[oc];
-    for (int d = 0; d < 7; ++d) o[16 + d] = nfilt[d];
-    P.b_fe.assign(4, 0.f);  // unused for v4
-
-    P.w_rec.assign(cvad::kV4RecStreamFloats, 0.f);
-    P.b_rec.assign(512, 0.f);
-    const float *W[2] = {l1w, l2w}, *R[2] = {l1r, l2r}, *B[2] = {l1b, l2b};
-    for (int l = 0; l < 2; ++l)
-        for (int n = 0; n < 256; ++n) {
-            const int unit = n >> 2, gate = n & 3;
-            const int row = gate * 64 + unit;  // ONNX order i,o,f,c
-            for (int k = 0; k < 64; ++k) {
-                P.w_rec[(size_t)l * 32768 + k * 256 + n] = W[l][row * 64 + k];
-                P.w_rec[(size_t)l * 32768 + (64 + k) * 256 + n] = R[l][row * 64 + k];
-            }
-            P.b_rec[l * 256 + n] = B[l][row] + B[l][256 + row];
-        }
-    P.w_dec.resize(65);
-    std::memcpy(P.w_dec.data(), decw, 64 * 4);
-    P.w_dec[64] = decb[0];
-    return P;
-}
-
 template <typename T>
 int upload(cvad_engine *e, T **dst, const std::vector<T> &src) {
     CU_TRY(e, cudaMalloc(reinterpret_cast<void **>(dst), src.size() * sizeof(T)));
@@ -592,67 +214,27 @@ int validate_args(cvad_engine *e, const cvad_step_args *a) {
     return CVAD_OK;
 }
 
-// R^T[m][n] of scipy.signal.resample(x[N_in] -> 512), float64 closed form rounded to float32
-// (formula and the two Nyquist rules: cvad_resample.cuh header).
-void build_resample_rt(int n_in, std::vector<float> &rt) {
-    const int num = 512;
-    const double PI = 3.14159265358979323846;
-    const int K = std::min(num, n_in) / 2;
-    rt.assign((size_t)n_in * num, 0.f);
-    for (int m = 0; m < n_in; ++m)
-        for (int n = 0; n < num; ++n) {
-            // theta/2 = pi (n/num - m/n_in), reduced with exact integer arithmetic
-            const long long L = (long long)num * n_in;
-            long long r = ((long long)n * n_in - (long long)m * num) % L;
-            if (r < 0) r += L;
-            const double half = PI * (double)r / (double)L;  // in [0, pi)
-            double dk;
-            if (r == 0) dk = 2.0 * K - 1.0;
-            else dk = std::sin((2.0 * K - 1.0) * half) / std::sin(half);
-            double nyq;
-            if (n_in > num) nyq = 2.0 * std::cos(PI * (double)(((long long)num * m) % (2LL * n_in)) / (double)n_in) *
-                                  ((n & 1) ? -1.0 : 1.0);
-            else nyq = std::cos(2.0 * K * half);
-            rt[(size_t)m * num + n] = (float)((dk + nyq) / (double)n_in);
-        }
-}
-
-// Enqueue the two kernels.  Every pointer in `a` is a DEVICE pointer here.
+// A source rate's resampling operator, built and uploaded on its first use: R^T for resample_kernel (FP32 math), both
+// tile forms for resample_tc_kernel (TC and TC16 math)
 int ensure_rt(cvad_engine *e, int src_rate, cudaStream_t stream) {
-    const int ri = rate_index(src_rate), n_in = rate_n_in(src_rate);
+    const int ri = rate_index(src_rate);
     if (e->rs_rt[ri]) return CVAD_OK;
-    std::vector<float> rt;
-    build_resample_rt(n_in, rt);
+    const std::vector<float> rt = build_resample_operator(rate_n_in(src_rate)).rt;
     CU_TRY(e, cudaMalloc(reinterpret_cast<void **>(&e->rs_rt[ri]), rt.size() * sizeof(float)));
     CU_TRY(e, cudaMemcpyAsync(e->rs_rt[ri], rt.data(), rt.size() * sizeof(float), cudaMemcpyHostToDevice, stream));
     CU_TRY(e, cudaStreamSynchronize(stream));
     return CVAD_OK;
 }
 
-// R as BF16x3 tiles for resample_tc_kernel: K block kb-major, then output block (128 samples), then part
 int ensure_rt_tc(cvad_engine *e, int src_rate, cudaStream_t stream) {
-    const int ri = rate_index(src_rate), n_in = rate_n_in(src_rate);
+    const int ri = rate_index(src_rate);
     if (e->rs_tc[ri]) return CVAD_OK;
-    std::vector<float> rt;
-    build_resample_rt(n_in, rt);            // R^T [n_in][512]
-    std::vector<unsigned char> tiles;
-    tiles.reserve((size_t)512 * n_in * 6);
-    for (int kb = 0; kb < n_in / 64; ++kb)
-        for (int blk = 0; blk < 4; ++blk)
-            emit_tiles(tiles, 128, kb * 64, [&](int r, int m) { return rt[(size_t)m * 512 + blk * 128 + r]; });
-    CU_TRY(e, cudaMalloc(reinterpret_cast<void **>(&e->rs_tc[ri]), tiles.size()));
-    CU_TRY(e, cudaMemcpyAsync(e->rs_tc[ri], tiles.data(), tiles.size(), cudaMemcpyHostToDevice, stream));
-    // the FP16 two-part form of the same operator, scaled so that its largest entry lies in [2^14, 2^15)
-    float mx = 0.f;
-    for (float v : rt) mx = std::max(mx, std::fabs(v));
-    const float sw = pow2_scale_for(mx, &e->rs_h_inv[ri]);
-    std::vector<unsigned char> th;
-    th.reserve((size_t)512 * n_in * 4);
-    for (int kb = 0; kb < n_in / 64; ++kb)
-        for (int blk = 0; blk < 4; ++blk)
-            emit_tiles_h(th, 128, kb * 64, sw, [&](int r, int m) { return rt[(size_t)m * 512 + blk * 128 + r]; });
-    CU_TRY(e, cudaMalloc(reinterpret_cast<void **>(&e->rs_h[ri]), th.size()));
-    CU_TRY(e, cudaMemcpyAsync(e->rs_h[ri], th.data(), th.size(), cudaMemcpyHostToDevice, stream));
+    const ResampleOperator op = build_resample_operator(rate_n_in(src_rate));
+    CU_TRY(e, cudaMalloc(reinterpret_cast<void **>(&e->rs_tc[ri]), op.tc.size()));
+    CU_TRY(e, cudaMemcpyAsync(e->rs_tc[ri], op.tc.data(), op.tc.size(), cudaMemcpyHostToDevice, stream));
+    CU_TRY(e, cudaMalloc(reinterpret_cast<void **>(&e->rs_h[ri]), op.tc16.size()));
+    CU_TRY(e, cudaMemcpyAsync(e->rs_h[ri], op.tc16.data(), op.tc16.size(), cudaMemcpyHostToDevice, stream));
+    e->rs_h_inv[ri] = op.inv;
     CU_TRY(e, cudaStreamSynchronize(stream));
     return CVAD_OK;
 }
@@ -703,6 +285,7 @@ __global__ void downmix_kernel(const void *audio, int pcm, long long stride, int
     }
 }
 
+// Enqueue the step's kernels.  Every pointer in `a` is a DEVICE pointer here.
 // `chain` (cvad_step_device on a fused one-frame step): the caller enqueued no memset; see cvad_engine::d_evctr.
 // `input_out` != nullptr (cvad_debug_input): run the input stages only, their output buffer filled with NaN first, and
 // return the device address of the mono 16 kHz samples the model kernels would read in *input_out.
@@ -777,7 +360,6 @@ int launch_step(cvad_engine *e, const cvad_step_args *a, unsigned int *d_status,
         r.n_streams = a->n_streams; r.n_stiles = n_stiles; r.max_frames = a->max_frames; r.n_frames = a->n_frames;
         r.out = static_cast<float *>(e->d_res.p);
         const int grid_rs = std::min(a->max_frames * n_stiles, e->num_sms);
-        const bool rs_tc = e->math != CVAD_MATH_FP32;
         // fewer 64-stream tiles than SMs: share a tile's four output blocks among 2 or 4 CTAs
         const int rs_tiles = a->max_frames * ((a->n_streams + cvad::tc5::kRsTcTile - 1) / cvad::tc5::kRsTcTile);
         // (mixed-rate steps launch once per rate over that rate's share of the streams: assume an even share)
@@ -785,29 +367,22 @@ int launch_step(cvad_engine *e, const cvad_step_args *a, unsigned int *d_status,
         const int rs_share = (rs_tiles + n_rates - 1) / n_rates;
         r.osplit = 4 * rs_share <= e->num_sms ? 4 : (2 * rs_share <= e->num_sms ? 2 : 1);
         const int grid_rs_tc = std::min(rs_tiles * r.osplit, e->num_sms);
-        const bool rs_fft = e->resampler == CVAD_RESAMPLE_FFT;
-        auto launch_rs_fft = [&](int n_in) {
-            // one warp per two frames; 1 CTA per SM (shared memory), grid = enough CTAs for the launch's upper bound of units
-            const long long units = (long long)a->max_frames * ((a->n_streams + 1) / 2);
-            const double2 *T = e->fft_T;
-            if (n_in == 256) {
-                const int g = (int)std::min<long long>((units + cvad::RsFft<1>::WPC - 1) / cvad::RsFft<1>::WPC, e->num_sms);
-                cvad::resample_fft_kernel<1><<<g, cvad::RsFft<1>::WPC * 32, cvad::RsFft<1>::kSmem, stream>>>(r, T);
-            } else if (n_in == 768) {
-                const int g = (int)std::min<long long>((units + cvad::RsFft<3>::WPC - 1) / cvad::RsFft<3>::WPC, e->num_sms);
-                cvad::resample_fft_kernel<3><<<g, cvad::RsFft<3>::WPC * 32, cvad::RsFft<3>::kSmem, stream>>>(r, T);
-            } else {
-                const int g = (int)std::min<long long>((units + cvad::RsFft<6>::WPC - 1) / cvad::RsFft<6>::WPC, e->num_sms);
-                cvad::resample_fft_kernel<6><<<g, cvad::RsFft<6>::WPC * 32, cvad::RsFft<6>::kSmem, stream>>>(r, T);
-            }
-        };
-        if (!mixed) {
-            r.n_in = rate_n_in(a->src_rate);
-            if (rs_fft) {
-                launch_rs_fft(r.n_in);
-            } else if (rs_tc) {
-                if ((rc = ensure_rt_tc(e, a->src_rate, stream))) return rc;
-                const int ri = rate_index(a->src_rate);
+        // run source rate `src_rate`'s resampler over `r`: every stream of the step, or the streams of r.list
+        auto launch_rs = [&](int src_rate) -> int {
+            const int ri = rate_index(src_rate);
+            r.n_in = rate_n_in(src_rate);
+            if (e->resampler == CVAD_RESAMPLE_FFT) {
+                // one warp per two frames; 1 CTA per SM (shared memory), grid = enough CTAs for the launch's upper bound of units
+                const long long units = (long long)a->max_frames * ((a->n_streams + 1) / 2);
+                auto fft = [&](auto kernel, int wpc, int smem) {
+                    const int g = (int)std::min<long long>((units + wpc - 1) / wpc, e->num_sms);
+                    kernel<<<g, wpc * 32, smem, stream>>>(r, e->fft_T);
+                };
+                if (r.n_in == 256) fft(cvad::resample_fft_kernel<1>, cvad::RsFft<1>::WPC, cvad::RsFft<1>::kSmem);
+                else if (r.n_in == 768) fft(cvad::resample_fft_kernel<3>, cvad::RsFft<3>::WPC, cvad::RsFft<3>::kSmem);
+                else fft(cvad::resample_fft_kernel<6>, cvad::RsFft<6>::WPC, cvad::RsFft<6>::kSmem);
+            } else if (e->math != CVAD_MATH_FP32) {
+                if ((rc = ensure_rt_tc(e, src_rate, stream))) return rc;
                 if (e->math == CVAD_MATH_TC16)
                     cvad::tc5::resample_tc_kernel<true><<<grid_rs_tc, cvad::tc5::kThreadsTC, cvad::tc5::kRsTcSmem, stream>>>(
                         r, e->rs_h[ri], e->rs_h_inv[ri]);
@@ -815,12 +390,16 @@ int launch_step(cvad_engine *e, const cvad_step_args *a, unsigned int *d_status,
                     cvad::tc5::resample_tc_kernel<false><<<grid_rs_tc, cvad::tc5::kThreadsTC, cvad::tc5::kRsTcSmem, stream>>>(
                         r, e->rs_tc[ri], 1.f);
             } else {
-                if ((rc = ensure_rt(e, a->src_rate, stream))) return rc;
-                r.rt = e->rs_rt[rate_index(a->src_rate)];
+                if ((rc = ensure_rt(e, src_rate, stream))) return rc;
+                r.rt = e->rs_rt[ri];
                 cvad::resample_kernel<<<grid_rs, cvad::kThreads, cvad::kRsSmemBytes, stream>>>(r);
             }
             CU_TRY(e, cudaGetLastError());
             e->launches++;
+            return CVAD_OK;
+        };
+        if (!mixed) {
+            if ((rc = launch_rs(a->src_rate))) return rc;
         } else {
             // one launch per source rate over that rate's stream list (built on the device: no host round trip)
             const size_t n = (size_t)a->n_streams;
@@ -835,26 +414,9 @@ int launch_step(cvad_engine *e, const cvad_step_args *a, unsigned int *d_status,
             static const int kRates[3] = {8000, 24000, 48000};
             for (int ri = 0; ri < 3; ++ri) {
                 if (!(rates_mask & (1u << ri))) continue;
-                r.n_in = rate_n_in(kRates[ri]);
                 r.list = lists + (size_t)ri * n;
                 r.count = counts + ri;
-                if (rs_fft) {
-                    launch_rs_fft(r.n_in);
-                } else if (rs_tc) {
-                    if ((rc = ensure_rt_tc(e, kRates[ri], stream))) return rc;
-                    if (e->math == CVAD_MATH_TC16)
-                        cvad::tc5::resample_tc_kernel<true><<<grid_rs_tc, cvad::tc5::kThreadsTC, cvad::tc5::kRsTcSmem, stream>>>(
-                            r, e->rs_h[ri], e->rs_h_inv[ri]);
-                    else
-                        cvad::tc5::resample_tc_kernel<false><<<grid_rs_tc, cvad::tc5::kThreadsTC, cvad::tc5::kRsTcSmem, stream>>>(
-                            r, e->rs_tc[ri], 1.f);
-                } else {
-                    if ((rc = ensure_rt(e, kRates[ri], stream))) return rc;
-                    r.rt = e->rs_rt[ri];
-                    cvad::resample_kernel<<<grid_rs, cvad::kThreads, cvad::kRsSmemBytes, stream>>>(r);
-                }
-                CU_TRY(e, cudaGetLastError());
-                e->launches++;
+                if ((rc = launch_rs(kRates[ri]))) return rc;
             }
             if (rates_mask & 8u) {
                 r.n_in = 512;
@@ -1502,7 +1064,7 @@ int cvad_create(const float *weights, size_t n_weight_floats, int model_version,
                   : (m && std::strcmp(m, "fp32") == 0) || !e->v4_fft_ok ? CVAD_MATH_FP32 : CVAD_MATH_FFT;
     }
     {
-        V5Packed P = model_version == CVAD_MODEL_V5 ? pack_v5(weights) : pack_v4(weights);
+        Fp32Packed P = model_version == CVAD_MODEL_V5 ? pack_v5(weights) : pack_v4(weights);
         int rc;
         if ((rc = upload(e, &e->w_fe, P.w_fe)) || (rc = upload(e, &e->b_fe, P.b_fe)) ||
             (rc = upload(e, &e->w_rec, P.w_rec)) || (rc = upload(e, &e->b_rec, P.b_rec)) ||
